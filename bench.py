@@ -25,6 +25,11 @@ One JSON line is printed by rank 0:
              compared byte for byte with the ndev = 1 result
 --impl reference times the reference's CPU algorithm (the oracle port: the reference itself is Python 2 and cannot run
 here) with multiprocessing on all host cores, on a bounded sample per step.
+
+--dump-outputs DIR writes what rank 0's last timed step of `value` returned, on a fixed sample of DUMP_ROWS rows (the same
+rows in every run with the same --rows): DIR/out.npy (rows x 32 bytes of the encoded shared secret, float32), DIR/status.npy
+(float32) and DIR/rows.npy (the sampled row indices, float64), 35 MiB in all.  The inputs are seeded, so two builds can be
+compared output for output.
 """
 import argparse
 import json
@@ -56,6 +61,7 @@ INV_SAVING = 1504 - (1504 // INV_ROWS + 3 * 48)
 PREP_SAVING = {"windowed": 192, "endo": 192 + 336}
 BYTES_PER_ROW = 96              # 32 scalar + 32 point + 32 out
 WORKLOAD = "cfg3 variable-base DH (decode+validate+[392]P+[k]Q+inversion+encode), 2^20 (scalar, encoded point) rows per GPU"
+DUMP_ROWS = 1 << 18             # --dump-outputs sample: 2^18 x 33 float32 + 2^18 float64 = 35 MiB
 
 
 def shard_bounds(n, world, rank):
@@ -71,6 +77,17 @@ def make_inputs(fq, rows, rank):
     kp = np.random.default_rng(4 + 1000 * rank).integers(0, 256, (rows, 32), np.uint8)
     pub = fq.MUL_base(kp)
     return k, pub
+
+
+def dump_outputs(path, out, status):
+    """Writes a fixed, seeded sample of DUMP_ROWS rows of one step's outputs (all rows when there are fewer) as float32 .npy
+    files, with the sampled row indices."""
+    rows = len(status)
+    idx = np.arange(rows) if rows <= DUMP_ROWS else np.sort(np.random.default_rng(0).choice(rows, DUMP_ROWS, replace=False))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "out.npy"), out[idx].astype(np.float32))
+    np.save(os.path.join(path, "status.npy"), status[idx].astype(np.float32))
+    np.save(os.path.join(path, "rows.npy"), idx.astype(np.float64))
 
 
 class ClockSampler:
@@ -341,6 +358,7 @@ def measure_inproc(fq, world, algorithm, quick=False):
 
 
 def main():
+    sys.dont_write_bytecode = True      # the tree may be read-only, and a benchmark run leaves nothing behind in it
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=10)
@@ -353,7 +371,12 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the cfg 2 / 4 / 5 measurements and the in-process multi-GPU phase")
     ap.add_argument("--quick", action="store_true", help="developer runs: small cfg 2 / 4 / in-process batches")
     ap.add_argument("--verify-rows", type=int, default=-1, help="rows of rank 0's batch compared bit for bit with the C oracle after the timed regions (default all; 0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a fixed sample of rank 0's outputs of the last timed step to DIR/*.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     out = _quiet_stdout()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -537,6 +560,8 @@ def main():
                                  "note": "fourq_b200.DH(k, B) on plain numpy arrays, outputs allocated by the call; the engine stages pageable operands through pinned buffers on its own threads"},
                 "gpu_launches": 3 * args.steps,
                 "roofline": roofline, "cpu_baseline": cpu, "parity": parity, "configs": configs, "inproc": inproc}
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, out_dev, st_dev)
     barrier()
     if dist is not None:
         dist.destroy_process_group()
