@@ -10,7 +10,7 @@
 //   drainer  (one per GPU)  waits for each chunk's completion event in order, copies results that were staged for a
 //                           pageable destination into the caller's memory, collects the kernel time and frees the slot.
 //
-// Four stream slots per GPU (FQ_SLOTS) keep the staging and H2D of the chunks after next, the kernels of chunk c, a chunk queued
+// Four stream slots per GPU keep the staging and H2D of the chunks after next, the kernels of chunk c, a chunk queued
 // behind it (so that kernel tails overlap the next chunk's first kernel) and the D2H and host copy-out of chunk c-1 in flight.  Page-locked caller buffers (fq_host_alloc) are used directly in both directions.  Slot buffers,
 // events and streams are created once per GPU and grow on demand; fq_trim wipes and frees them.  There is no CPU
 // implementation of any operation here.
@@ -43,7 +43,7 @@
 
 namespace {
 
-constexpr int kSlots = 6;                        // stream slots created per GPU; slots_in_use() of them carry chunks
+constexpr int kSlots = 4;                        // stream slots per GPU = chunks in flight (see the top of this file)
 constexpr int kMaxDev = 16;
 constexpr int kOperands = 5;                      // a, b, c (inputs), out, status
 constexpr size_t kFlushBytes = 256u << 20;        // > 126 MB L2
@@ -65,25 +65,27 @@ int fail(int code, const char* fmt, ...) {
 
 // ---------------------------------------------------------------- operations
 
-// bytes per row of each operand of an operation; chunk_rows = rows of a full pipeline chunk
-struct OpDesc { int op; int in_bytes[3]; int out_bytes; bool status; size_t chunk_rows; };
-
+// rows by which the chunk schedule rounds: ramp-down chunks, stolen pieces, speed-weighted slices and the half chunks of staged calls
+constexpr size_t kRowQuant = 128;
 // rows per full pipeline chunk of the variable-base DH ops: a whole number of waves of k_dh_ladder (2 CTAs x 128 rows per SM)
-// and of k_dh_prep (3 per SM) keeps the tail of each chunk short; FQ_DH_CHUNK_ROWS overrides it (tuning knob, read once,
-// rounded down to a multiple of 128).
-size_t dh_chunk_rows() {
-  static const size_t v = [] {
-    const char* e = getenv("FQ_DH_CHUNK_ROWS");
-    const long long x = e ? atoll(e) : 0;
-    return x >= 128 ? (size_t)x / 128 * 128 : (size_t)148 * 2 * 128 * 12;      // 454,656 rows = 12 waves of k_dh_ladder, 8 of k_dh_prep
-  }();
-  return v;
-}
-// FQ_PIPELINE_RAMP=0 disables the ramped chunk schedule (all chunks full size)
-bool ramp_enabled() {
-  static const bool v = [] { const char* e = getenv("FQ_PIPELINE_RAMP"); return !(e && e[0] == '0'); }();
-  return v;
-}
+// and of k_dh_prep (3 per SM) keeps the tail of each chunk short
+constexpr size_t kDhChunkRows = (size_t)148 * 2 * 128 * 12;      // 454,656 rows = 12 waves of k_dh_ladder, 8 of k_dh_prep
+// k_comb keeps 2 CTAs of 256 rows resident per SM, each walking over tiles: 148 x 2 x 256 x 4 rows = 4 full tiles per CTA
+constexpr size_t kCombChunkRows = (size_t)148 * 2 * 256 * 4;
+
+// device scratch an operation's kernels hand data through: none, the variable-base DH layout (table, digit register,
+// projective result), the projective result the fixed-base kernels hand to k_dh_finish, or the X25519 ladder's (x2, z2)
+enum Scratch { SCRATCH_NONE, SCRATCH_DH, SCRATCH_FIXED_BASE, SCRATCH_X25519 };
+
+// Everything the engine knows about an operation apart from its kernels (launch):
+//   bytes per row of each operand, chunk_rows = rows of a full pipeline chunk, the scratch its kernels need;
+//   rate_class >= 0: big multi-GPU calls adapt their slices to the measured speed of each GPU (on a host where some GPUs reach
+//   the caller's memory more slowly than others, equal slices end with the slowest GPU); ops of one class share the measurement;
+//   var_dh: a variable-base DH op (three kernels; half chunks for staged operands, per-kernel timing in fq_dev_run3).
+struct OpDesc {
+  int op; int in_bytes[3]; int out_bytes; bool status; size_t chunk_rows;
+  Scratch scratch = SCRATCH_NONE; int rate_class = -1; bool var_dh = false;
+};
 
 OpDesc describe(int op) {
   const size_t M = (size_t)1 << 20;
@@ -99,14 +101,15 @@ OpDesc describe(int op) {
     case FQ_DEVOP_DECODE: case FQ_DEVOP_DECODE_SPEC: return {op, {32, 0, 0}, 64, true, M / 4};
     case FQ_DEVOP_ENCODE: return {op, {64, 0, 0}, 32, false, M};
     case FQ_DEVOP_ON_CURVE: return {op, {64, 0, 0}, 1, false, M};
-    case FQ_DEVOP_DH: case FQ_DEVOP_DH_ENDO: return {op, {32, 32, 0}, 32, true, dh_chunk_rows()};
-    case FQ_DEVOP_DH_AFFINE: case FQ_DEVOP_DH_ENDO_AFFINE: return {op, {32, 64, 0}, 64, true, dh_chunk_rows()};
-    case FQ_DEVOP_DH_BASE: case FQ_DEVOP_DH_ENDO_BASE: return {op, {32, 0, 0}, 32, true, M / 8};
-    case FQ_DEVOP_MUL_BASE: case FQ_DEVOP_MUL_ENDO_BASE: return {op, {32, 0, 0}, 32, false, M / 8};
-    // k_comb keeps 2 CTAs of 256 rows resident per SM, each walking over tiles: 148 x 2 x 256 x 4 rows = 4 full tiles per CTA
-    case FQ_DEVOP_DH_BASE_COMB: return {op, {32, 0, 0}, 32, true, (size_t)148 * 2 * 256 * 4};
-    case FQ_DEVOP_MUL_BASE_COMB: return {op, {32, 0, 0}, 32, false, (size_t)148 * 2 * 256 * 4};
-    case FQ_DEVOP_X25519: return {op, {32, 32, 0}, 32, false, M / 8};
+    case FQ_DEVOP_DH: return {op, {32, 32, 0}, 32, true, kDhChunkRows, SCRATCH_DH, 0, true};
+    case FQ_DEVOP_DH_AFFINE: return {op, {32, 64, 0}, 64, true, kDhChunkRows, SCRATCH_DH, 0, true};
+    case FQ_DEVOP_DH_ENDO: return {op, {32, 32, 0}, 32, true, kDhChunkRows, SCRATCH_DH, 1, true};
+    case FQ_DEVOP_DH_ENDO_AFFINE: return {op, {32, 64, 0}, 64, true, kDhChunkRows, SCRATCH_DH, 1, true};
+    case FQ_DEVOP_DH_BASE: case FQ_DEVOP_DH_ENDO_BASE: return {op, {32, 0, 0}, 32, true, M / 8, SCRATCH_FIXED_BASE};
+    case FQ_DEVOP_MUL_BASE: case FQ_DEVOP_MUL_ENDO_BASE: return {op, {32, 0, 0}, 32, false, M / 8, SCRATCH_FIXED_BASE};
+    case FQ_DEVOP_DH_BASE_COMB: return {op, {32, 0, 0}, 32, true, kCombChunkRows, SCRATCH_FIXED_BASE, 2};
+    case FQ_DEVOP_MUL_BASE_COMB: return {op, {32, 0, 0}, 32, false, kCombChunkRows, SCRATCH_FIXED_BASE, 2};
+    case FQ_DEVOP_X25519: return {op, {32, 32, 0}, 32, false, M / 8, SCRATCH_X25519};
     case FQ_DEVOP_F25519_BASE + FQ_FP_MUL: case FQ_DEVOP_F25519_BASE + FQ_FP_ADD: case FQ_DEVOP_F25519_BASE + FQ_FP_SUB: return {op, {32, 32, 0}, 32, false, M};
     case FQ_DEVOP_F25519_BASE + FQ_FP_SQR: return {op, {32, 0, 0}, 32, false, M};
     case FQ_DEVOP_F25519_BASE + FQ_FP_INV: return {op, {32, 0, 0}, 32, false, M / 4};
@@ -114,27 +117,13 @@ OpDesc describe(int op) {
   }
 }
 int operand_bytes(const OpDesc& d, int w) { return w < 3 ? d.in_bytes[w] : w == 3 ? d.out_bytes : (d.status ? 1 : 0); }
-
-bool is_dh_op(int op) { return op == FQ_DEVOP_DH || op == FQ_DEVOP_DH_AFFINE || op == FQ_DEVOP_DH_ENDO || op == FQ_DEVOP_DH_ENDO_AFFINE; }
-// fixed-base ops: their kernels hand (X, Y, Z) to k_dh_finish through a small scratch
-bool is_comb_op(int op) {
-  return op == FQ_DEVOP_DH_BASE_COMB || op == FQ_DEVOP_MUL_BASE_COMB || op == FQ_DEVOP_DH_BASE || op == FQ_DEVOP_MUL_BASE ||
-         op == FQ_DEVOP_DH_ENDO_BASE || op == FQ_DEVOP_MUL_ENDO_BASE;
-}
-bool needs_scratch(int op) { return is_dh_op(op) || is_comb_op(op) || op == FQ_DEVOP_X25519; }
-size_t scratch_bytes(int op, size_t rows) {
-  return is_comb_op(op) ? fqk_comb_scratch_bytes(rows) : op == FQ_DEVOP_X25519 ? fqk_x25519_scratch_bytes(rows) : fqk_dh_scratch_bytes(rows);
-}
-
-// Operations whose big multi-GPU calls adapt their slices to the measured speed of each GPU (FQ_ADAPT=0: always equal slices).
-// On a host where some GPUs reach the caller's memory more slowly than others, equal slices end with the slowest GPU.
-int rate_class(int op) {
-  static const bool on = [] { const char* e = getenv("FQ_ADAPT"); return !(e && e[0] == '0'); }();
-  if (!on) return -1;
-  if (op == FQ_DEVOP_DH || op == FQ_DEVOP_DH_AFFINE) return 0;
-  if (op == FQ_DEVOP_DH_ENDO || op == FQ_DEVOP_DH_ENDO_AFFINE) return 1;
-  if (op == FQ_DEVOP_MUL_BASE_COMB || op == FQ_DEVOP_DH_BASE_COMB) return 2;
-  return -1;
+size_t scratch_bytes(Scratch k, size_t rows) {
+  switch (k) {
+    case SCRATCH_DH: return fqk_dh_scratch_bytes(rows);
+    case SCRATCH_FIXED_BASE: return fqk_comb_scratch_bytes(rows);
+    case SCRATCH_X25519: return fqk_x25519_scratch_bytes(rows);
+    default: return 0;
+  }
 }
 
 int strict_mode() {
@@ -161,17 +150,13 @@ struct CallWork {
   std::mutex mu;
   struct Range { size_t lo, hi; bool ramp; };
   std::vector<Range> r;               // rows of each slice not yet handed out
-  size_t full = 0, small = 0, quant = 128;
-  bool steal = true, abort = false;
+  size_t full = 0, small = 0;
+  bool abort = false;
   // share: optional relative speeds of the GPUs (rows per ms of their last calls); null or incomplete -> equal slices
   void init(size_t n, int ndev, size_t full_rows, const double* share = nullptr) {
     full = full_rows;
     small = full / 8 >= 16384 ? full / 8 : 16384;
     if (small > full) small = full;
-    static const size_t q_env = [] { const char* e = getenv("FQ_CHUNK_QUANT"); long long x = e ? atoll(e) : 0; return x >= 128 ? (size_t)x / 128 * 128 : (size_t)128; }();
-    quant = q_env <= small ? q_env : 128;
-    static const bool steal_on = [] { const char* e = getenv("FQ_STEAL"); return !(e && e[0] == '0'); }();
-    steal = steal_on;
     const size_t per = (n + (size_t)ndev - 1) / (size_t)ndev;
     double total = 0;
     bool weighted = share != nullptr && ndev > 1 && n >= (size_t)ndev * 2 * full;
@@ -190,11 +175,11 @@ struct CallWork {
     for (int i = 0; i < ndev; i++) {
       size_t len = per;
       if (weighted) {
-        len = (size_t)((double)n * f[i] / fsum) / 128 * 128;
+        len = (size_t)((double)n * f[i] / fsum) / kRowQuant * kRowQuant;
         if (i == ndev - 1) len = n - lo;
       }
       const size_t hi = lo + len < n ? lo + len : n;
-      r.push_back({lo, i == ndev - 1 && weighted ? n : hi, ramp_enabled() && hi - lo > 2 * small});
+      r.push_back({lo, i == ndev - 1 && weighted ? n : hi, hi - lo > 2 * small});
       lo = hi;
     }
   }
@@ -208,20 +193,19 @@ struct CallWork {
       size_t sz = full;
       if (own.ramp) { sz = small; for (int t = 0; t < taken && sz < full; t++) sz = sz * 2 < full ? sz * 2 : full; }
       size_t n = sz < left ? sz : left;
-      if (own.ramp && left > small && left <= 2 * n) {              // ramp down by halves, in units of `quant` rows
-        n = (left / 2 + quant - 1) / quant * quant;
+      if (own.ramp && left > small && left <= 2 * n) {              // ramp down by halves
+        n = (left / 2 + kRowQuant - 1) / kRowQuant * kRowQuant;
         if (n > full) n = full;
         if (n > left) n = left;
       }
       *r0 = own.lo; *rows = n; own.lo += n;
       return true;
     }
-    if (!steal) return false;
     size_t best = r.size(), most = 0;
     for (size_t j = 0; j < r.size(); j++) if (r[j].hi - r[j].lo > most) { most = r[j].hi - r[j].lo; best = j; }
     if (best == r.size()) return false;
     size_t n = most;                                                 // a victim's last piece goes whole; otherwise half of what it has left
-    if (most > small) { n = (most / 2 + 127) / 128 * 128; if (n > full) n = full; if (n > most) n = most; }
+    if (most > small) { n = (most / 2 + kRowQuant - 1) / kRowQuant * kRowQuant; if (n > full) n = full; if (n > most) n = most; }
     r[best].hi -= n; *r0 = r[best].hi; *rows = n;
     return true;
   }
@@ -230,13 +214,10 @@ struct CallWork {
 
 // ---------------------------------------------------------------- host copies of pageable operands
 
-// FQ_COPY_THREADS (1..4, default 3): threads that share one staging copy of a pageable operand.  One core moves 5-10 GB/s,
-// a B200 consumes the 64 B of inputs per DH row at ~6 GB/s and produces 33 B, so a single copying thread per direction is
-// on the critical path (measured: 68 / 73 / 75 M DH rows/s end to end with 1 / 2 / 3 threads before the other changes).
-int copy_threads() {
-  static const int v = [] { const char* e = getenv("FQ_COPY_THREADS"); int x = e ? atoi(e) : 3; return x < 1 ? 1 : x > 4 ? 4 : x; }();
-  return v;
-}
+// threads that share one staging copy of a pageable operand.  One core moves 5-10 GB/s, a B200 consumes the 64 B of inputs
+// per DH row at ~6 GB/s and produces 33 B, so a single copying thread per direction is on the critical path (measured: 68 / 73 /
+// 75 M DH rows/s end to end with 1 / 2 / 3 threads before the other changes).
+constexpr int kCopyThreads = 3;
 // Makes the pages of a pageable OUTPUT buffer present and writable without touching their contents (MADV_POPULATE_WRITE,
 // Linux 5.14+; silently skipped where unsupported).  A freshly allocated result array (numpy.empty) otherwise takes its
 // ~8,000 first-touch page faults per 32 MiB inside the drainer's copies, on the critical path of the last chunks.  Called by
@@ -245,21 +226,13 @@ void populate_output(void* p, size_t bytes) {
 #ifndef MADV_POPULATE_WRITE
 #define MADV_POPULATE_WRITE 23
 #endif
-  static const bool enabled = [] { const char* e = getenv("FQ_POPULATE"); return !(e && e[0] == '0'); }();
-  if (!enabled || !p || bytes < ((size_t)1 << 20)) return;
+  if (!p || bytes < ((size_t)1 << 20)) return;
   const size_t page = (size_t)sysconf(_SC_PAGESIZE);
   uintptr_t lo = ((uintptr_t)p + page - 1) / page * page, hi = ((uintptr_t)p + bytes) / page * page;      // whole pages inside the buffer
-  static const bool huge = [] { const char* e = getenv("FQ_POPULATE_HUGE"); return !(e && e[0] == '0'); }();
-  if (huge && hi > lo) madvise((void*)lo, hi - lo, MADV_HUGEPAGE);       // where transparent huge pages are on request: 16 faults per 32 MiB instead of 8,192
+  if (hi > lo) madvise((void*)lo, hi - lo, MADV_HUGEPAGE);       // where transparent huge pages are on request: 16 faults per 32 MiB instead of 8,192
   const size_t step = (size_t)4 << 20;
   for (; lo < hi; lo += step)
     if (madvise((void*)lo, hi - lo < step ? hi - lo : step, MADV_POPULATE_WRITE) != 0) return;
-}
-// FQ_SLOTS (2..6, default 4): chunks in flight per GPU.  One is being computed, one is queued behind it (so that the tail of a
-// kernel overlaps the next chunk's first kernel), and the others are in host staging on their way in or out.
-int slots_in_use() {
-  static const int v = [] { const char* e = getenv("FQ_SLOTS"); int x = e ? atoi(e) : 4; return x < 2 ? 2 : x > kSlots ? kSlots : x; }();
-  return v;
 }
 // FQ_WIPE_AFTER_CALL=1: zero the staging buffers and the kernel scratch of a GPU when its slice of a call is done (they hold
 // scalars, tables of secret multiples, projective results and shared secrets until the next call overwrites them or fq_trim
@@ -274,11 +247,11 @@ bool trace_enabled() {
 }
 double now_ms() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 
-// memcpy split between the calling thread and up to three helper threads that sleep between copies
+// memcpy split between the calling thread and kCopyThreads - 1 helper threads that sleep between copies
 class CopyHelper {
  public:
   void copy(void* dst, const void* src, size_t bytes) {
-    const int parts = bytes >= ((size_t)1 << 20) ? copy_threads() : 1;
+    const int parts = bytes >= ((size_t)1 << 20) ? kCopyThreads : 1;
     if (parts == 1) { memcpy(dst, src, bytes); return; }
     const size_t per = (bytes / parts + 4095) / 4096 * 4096;
     {
@@ -406,8 +379,8 @@ int hbuf_reserve(Slot& s, int w, size_t bytes) {
   s.hcap[w] = bytes;
   return FQ_OK;
 }
-int scratch_reserve(Slot& s, int op, size_t rows) {
-  const size_t bytes = scratch_bytes(op, rows);
+int scratch_reserve(Slot& s, Scratch k, size_t rows) {
+  const size_t bytes = scratch_bytes(k, rows);
   if (bytes <= s.scratch_cap) return FQ_OK;
   tl_grew = true;
   if (s.scratch) CU(cudaFree(s.scratch));
@@ -506,7 +479,7 @@ int feed_slice(DevCtx& c, SliceJob* j) {
   size_t r0 = 0, rows = 0;
   tl_grew = false;
   for (int ci = 0; rc == FQ_OK && j->work->take(j->index, ci, &r0, &rows); ci++) {
-    const int si = ci % slots_in_use();
+    const int si = ci % kSlots;
     Slot& s = c.slot[si];
     const double tw0 = now_ms();
     { std::unique_lock<std::mutex> l(c.smu); c.scv.wait(l, [&] { return !s.busy; }); if (j->rc != FQ_OK) break; }     // a retired chunk failed: stop feeding
@@ -520,7 +493,7 @@ int feed_slice(DevCtx& c, SliceJob* j) {
         if ((e = dbuf_reserve(s, w, d.chunk_rows * wb)) != FQ_OK) return e;
         if (!j->pinned[w] && (e = hbuf_reserve(s, w, d.chunk_rows * wb)) != FQ_OK) return e;
       }
-      if (needs_scratch(d.op) && (e = scratch_reserve(s, d.op, d.chunk_rows)) != FQ_OK) return e;
+      if ((e = scratch_reserve(s, d.scratch, d.chunk_rows)) != FQ_OK) return e;
       for (int w = 0; w < 3; w++) {
         const int wb = d.in_bytes[w];
         if (!wb) continue;
@@ -553,15 +526,14 @@ int feed_slice(DevCtx& c, SliceJob* j) {
   j->grew = tl_grew;
   { std::unique_lock<std::mutex> l(c.smu); c.scv.wait(l, [&] { return j->outstanding == 0; }); }
   if (wipe_after_call()) {
-    for (int si = 0; si < slots_in_use(); si++) {
-      Slot& s = c.slot[si];
+    for (Slot& s : c.slot) {
       for (int w = 0; w < kOperands; w++) {
         if (s.dbuf[w]) cudaMemsetAsync(s.dbuf[w], 0, s.dcap[w], s.st);
         if (s.hbuf[w]) memset(s.hbuf[w], 0, s.hcap[w]);
       }
       if (s.scratch) cudaMemsetAsync(s.scratch, 0, s.scratch_cap, s.st);
     }
-    for (int si = 0; si < slots_in_use(); si++) cudaStreamSynchronize(c.slot[si].st);
+    for (Slot& s : c.slot) cudaStreamSynchronize(s.st);
   }
   return j->rc;
 }
@@ -645,11 +617,11 @@ int run_host(int op, const uint8_t* a, const uint8_t* b, const uint8_t* cbuf, ui
   OpDesc dj = d;
   // Staged (pageable) operands add two host copies to every chunk's trip; shorter chunks shorten what is exposed at both ends
   // of the pipeline: half the chunk for the variable-base DH ops (measured, one B200: 13.7 -> 12.8 ms per 2^20 rows).
-  if (!all_pinned && is_dh_op(op) && dj.chunk_rows >= 2 * 37888) dj.chunk_rows = dj.chunk_rows / 2 / 128 * 128;
+  if (!all_pinned && d.var_dh) dj.chunk_rows = dj.chunk_rows / 2 / kRowQuant * kRowQuant;
   const double t_call0 = now_ms();
   CallState cs;
   CallWork work;
-  const int rc_class = rate_class(op);
+  const int rc_class = d.rate_class;
   double share[kMaxDev] = {0};
   if (rc_class >= 0) for (int i = 0; i < ndev; i++) share[i] = ctx_of(base + i).rate[rc_class].load();
   work.init(n, ndev, dj.chunk_rows, rc_class >= 0 ? share : nullptr);
@@ -905,19 +877,18 @@ int fq_dev_run3(int op, int dev, const void* a, const void* b, const void* c, vo
   if ((op == FQ_DEVOP_FP2_INV || op == FQ_DEVOP_F25519_BASE + FQ_FP_INV) && a == out) return fail(FQ_ERR_ARG, "inv: out must not alias a (the prefix products are parked in out)");
   DevCtx& cx = *L.c;
   Slot& s = cx.slot[0];
-  const bool dh = is_dh_op(op);
   int rc;
-  if (needs_scratch(op) && (rc = scratch_reserve(s, op, n)) != FQ_OK) return rc;
+  if ((rc = scratch_reserve(s, d.scratch, n)) != FQ_OK) return rc;
   cudaEvent_t ph[4];
   for (int i = 0; i < 4; i++) CU(cudaEventCreate(&ph[i]));
   CU(cudaEventRecord(s.e0, s.st));
-  for (int i = 0; i < iters; i++) CU(launch(cx, op, a, b, c, out, status, n, s.st, s.scratch, (dh && i == iters - 1) ? ph : nullptr));
+  for (int i = 0; i < iters; i++) CU(launch(cx, op, a, b, c, out, status, n, s.st, s.scratch, (d.var_dh && i == iters - 1) ? ph : nullptr));
   CU(cudaEventRecord(s.e1, s.st));
   CU(cudaEventSynchronize(s.e1));
   float t = 0.f;
   CU(cudaEventElapsedTime(&t, s.e0, s.e1));
   tl_phase_ms[0] = tl_phase_ms[1] = tl_phase_ms[2] = 0.f;
-  if (dh && n > 0) for (int i = 0; i < 3; i++) CU(cudaEventElapsedTime(&tl_phase_ms[i], ph[i], ph[i + 1]));
+  if (d.var_dh && n > 0) for (int i = 0; i < 3; i++) CU(cudaEventElapsedTime(&tl_phase_ms[i], ph[i], ph[i + 1]));
   for (int i = 0; i < 4; i++) cudaEventDestroy(ph[i]);
   if (ms) *ms = t / iters;
   return FQ_OK;

@@ -207,13 +207,7 @@ cudaError_t fqk_encode(const void* xy, void* enc, size_t n, cudaStream_t s) {
   k_encode<<<grid_for(n, 256), 256, 0, s>>>(xy, enc, n);
   return cudaGetLastError();
 }
-size_t fqk_dh_scratch_bytes(size_t n) {
-  // kernels_dh.cuh: (64 table + 2 digit-register + 6 result) quads of 16 B and one meta word per row, rows padded to 128,
-  // at most 2^22 rows per launch group
-  size_t rows = n < ((size_t)1 << 22) ? n : ((size_t)1 << 22);
-  size_t npad = (rows + 127) / 128 * 128;
-  return npad * (72 * 16 + 4);
-}
+size_t fqk_dh_scratch_bytes(size_t n) { return dh_scratch_bytes(n < FQ_DH_MAX_BATCH ? n : FQ_DH_MAX_BATCH); }
 cudaError_t fqk_dh(int affine, int endo, int strict, const void* k, const void* pt, void* out, void* status, size_t n, void* scratch, cudaStream_t s, cudaEvent_t* ev) {
   if (n == 0) return cudaSuccess;
   return endo ? fqk_dh_endo(affine, strict, k, pt, out, status, n, scratch, s, ev) : fqk_dh_windowed(affine, strict, k, pt, out, status, n, scratch, s, ev);

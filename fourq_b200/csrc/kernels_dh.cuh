@@ -20,24 +20,16 @@
 #include "kio.cuh"
 #include "batchinv.cuh"
 
-#define FQ_DH_THREADS 128
 #define FQ_DH_SMEM (56 * 16 * FQ_DH_THREADS)       // 7 table entries x 8 quads x 16 B per thread = 112 KiB per CTA
 
 // ---------------------------------------------------------------- the three-kernel pipeline
 
-#define FQ_DH_SCRATCH_QUADS (64 + 2 + 6)             // table | digit register | (X, Y, Z), 16 B each
-#define FQ_DH_MAX_BATCH ((size_t)1 << 22)            // rows per launch group (keeps the u32 table indices in range)
-
-// scratch of one batch: npad rows (a multiple of 128); every array is [component][row] so that warps move 512 B lines
+// scratch of one batch (sized in kernels.h): npad rows, a multiple of FQ_DH_THREADS
 struct DhScratch { uint4* tab; uint4* plan; uint4* R; u32* meta; size_t npad; };
 
-static inline size_t dh_scratch_bytes(size_t rows) {
-  size_t npad = (rows + FQ_DH_THREADS - 1) / FQ_DH_THREADS * FQ_DH_THREADS;
-  return npad * (FQ_DH_SCRATCH_QUADS * 16 + 4);
-}
 static inline DhScratch dh_scratch_view(void* base, size_t rows) {
   DhScratch sc;
-  sc.npad = (rows + FQ_DH_THREADS - 1) / FQ_DH_THREADS * FQ_DH_THREADS;
+  sc.npad = dh_scratch_npad(rows);
   sc.tab = reinterpret_cast<uint4*>(base); sc.plan = sc.tab + 64 * sc.npad; sc.R = sc.plan + 2 * sc.npad;
   sc.meta = reinterpret_cast<u32*>(sc.R + 6 * sc.npad);
   return sc;
@@ -47,10 +39,7 @@ __device__ __forceinline__ void stq(uint4* p, const fp& a) { *p = make_uint4(a.v
 __device__ __forceinline__ fp ldq(const uint4* p) { uint4 w = *p; return fp_set(w.x, w.y, w.z, w.w); }
 
 // three CTAs per SM with the endomorphisms (a fourth would spill), four without (measured: 3.26 vs 3.47 ms, 2.15 vs 2.21 ms)
-#ifndef FQ_PREP_MINB_ENDO
-#define FQ_PREP_MINB_ENDO 3
-#endif
-template <bool AFFINE, bool ENDO> __global__ void __launch_bounds__(FQ_DH_THREADS, ENDO ? FQ_PREP_MINB_ENDO : 4)
+template <bool AFFINE, bool ENDO> __global__ void __launch_bounds__(FQ_DH_THREADS, ENDO ? 3 : 4)
 k_dh_prep(const void* __restrict__ k, const void* __restrict__ pt, DhScratch sc, size_t n) {
   const size_t row = (size_t)blockIdx.x * FQ_DH_THREADS + threadIdx.x;
   const size_t src = row < n ? row : n - 1;          // tail threads recompute the last row (their scratch slots exist)
@@ -66,10 +55,9 @@ k_dh_prep(const void* __restrict__ k, const void* __restrict__ pt, DhScratch sc,
   sc.meta[row] = D.plan.first | (st << 8);
 }
 
-#ifndef FQ_LADDER_MAXREG
-#define FQ_LADDER_MAXREG 255
-#endif
-template <bool ENDO, bool STRICT> __global__ void __maxnreg__(FQ_LADDER_MAXREG)
+// no register cap: every cap below the 248 registers of the strict loop measured slower, and the shared-memory table alone
+// limits the ladder to two CTAs per SM (DESIGN.md 6, profiles/r02_ladder_regcap.txt)
+template <bool ENDO, bool STRICT> __global__ void __maxnreg__(255)
 k_dh_ladder(DhScratch sc) {
   extern __shared__ uint4 smem[];
   const size_t row = (size_t)blockIdx.x * FQ_DH_THREADS + threadIdx.x;
@@ -102,14 +90,10 @@ k_dh_finish(DhScratch sc, void* __restrict__ out, unsigned char* __restrict__ st
 static inline unsigned dh_finish_grid(size_t rows) {
   return (unsigned)((((rows + FQ_BATCHINV_ROWS - 1) / FQ_BATCHINV_ROWS) + FQ_FIN_THREADS - 1) / FQ_FIN_THREADS);
 }
-// scratch of a producer that only hands (X, Y, Z) and a status word to k_dh_finish (the fixed-base comb kernel)
-static inline size_t fin_scratch_bytes(size_t rows) {
-  size_t npad = (rows + 255) / 256 * 256;
-  return npad * (6 * 16 + 4);
-}
+// scratch of a producer that only hands (X, Y, Z) and a status word to k_dh_finish (the fixed-base kernels; sized in kernels.h)
 static inline DhScratch fin_scratch_view(void* base, size_t rows) {
   DhScratch sc;
-  sc.npad = (rows + 255) / 256 * 256;
+  sc.npad = fin_scratch_npad(rows);
   sc.tab = nullptr; sc.plan = nullptr; sc.R = reinterpret_cast<uint4*>(base); sc.meta = reinterpret_cast<u32*>(sc.R + 6 * sc.npad);
   return sc;
 }
@@ -119,7 +103,7 @@ template <bool ENDO> static cudaError_t dh_init() {
   if (e != cudaSuccess) return e;
   return cudaFuncSetAttribute(k_dh_ladder<ENDO, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, FQ_DH_SMEM);
 }
-// scratch: dh_scratch_bytes(min(n, FQ_DH_MAX_BATCH)) bytes on the device.  ev: optional 4 events recorded around the three
+// scratch: fqk_dh_scratch_bytes(n) bytes on the device.  ev: optional 4 events recorded around the three
 // kernels of the (last) batch, for per-kernel timing.
 // strict: table selection by the strict scan instead of masked loads (dh.cuh)
 template <bool ENDO> static cudaError_t dh_launch(int affine, int strict, const void* k, const void* pt, void* out, void* status, size_t n, void* scratch,

@@ -25,11 +25,11 @@ __global__ void __launch_bounds__(64) k_x25519_finish(const uint4* __restrict__ 
   batch_invert<F25Ops>(io, FQ_BATCHINV_ROWS);
 }
 
-size_t fqk_x25519_scratch_bytes(size_t n) { return (n + 127) / 128 * 128 * 64; }
+size_t fqk_x25519_scratch_bytes(size_t n) { return x25519_scratch_bytes(n); }
 
 cudaError_t fqk_x25519(const void* k, const void* u, void* out, size_t n, void* scratch, cudaStream_t s) {
   if (n == 0) return cudaSuccess;
-  const size_t npad = (n + 127) / 128 * 128;
+  const size_t npad = x25519_scratch_npad(n);
   k_x25519<<<(unsigned)(npad / 128), 128, 0, s>>>(k, u, (uint4*)scratch, npad, n);
   const size_t groups = (n + FQ_BATCHINV_ROWS - 1) / FQ_BATCHINV_ROWS;
   k_x25519_finish<<<(unsigned)((groups + 63) / 64), 64, 0, s>>>((const uint4*)scratch, npad, out, n);

@@ -59,7 +59,7 @@ cudaError_t fqk_on_curve(const void* xy, void* ok, size_t n, cudaStream_t s) {
   mock_stream_enqueue(s, [=] { sim_on_curve((cu8)xy, (u8)ok, n); });
   return cudaSuccess;
 }
-size_t fqk_dh_scratch_bytes(size_t n) { size_t npad = (n + 127) / 128 * 128; return npad * (72 * 16 + 4); }
+size_t fqk_dh_scratch_bytes(size_t n) { return dh_scratch_bytes(n < FQ_DH_MAX_BATCH ? n : FQ_DH_MAX_BATCH); }
 cudaError_t fqk_dh(int affine, int endo, int, const void* k, const void* pt, void* out, void* status, size_t n, void* scratch, cudaStream_t s, cudaEvent_t* ev) {
   if (ev) cudaEventRecord(ev[0], s);
   mock_stream_enqueue(s, [=] {
@@ -70,7 +70,7 @@ cudaError_t fqk_dh(int affine, int endo, int, const void* k, const void* pt, voi
   if (ev) { cudaEventRecord(ev[1], s); cudaEventRecord(ev[2], s); cudaEventRecord(ev[3], s); }
   return cudaSuccess;
 }
-size_t fqk_comb_scratch_bytes(size_t n) { size_t npad = (n + 255) / 256 * 256; return npad * (6 * 16 + 4); }
+size_t fqk_comb_scratch_bytes(size_t n) { return fin_scratch_bytes(n < FQ_DH_MAX_BATCH ? n : FQ_DH_MAX_BATCH); }
 cudaError_t fqk_fixed_base(int dh, int endo, int, const void* k, void* out, void* status, size_t n, void* scratch, cudaStream_t s) {
   mock_stream_enqueue(s, [=] { memset(scratch, 0x11, fqk_comb_scratch_bytes(n)); sim_fixed_base(dh | (endo << 1), (cu8)k, (u8)out, (u8)status, n); });
   return cudaSuccess;
@@ -80,7 +80,7 @@ cudaError_t fqk_comb(int dh, int, const void*, const void* k, void* out, void* s
   mock_stream_enqueue(s, [=] { memset(scratch, 0x11, fqk_comb_scratch_bytes(n)); sim_comb(dh, (cu8)k, (u8)out, (u8)status, n); });
   return cudaSuccess;
 }
-size_t fqk_x25519_scratch_bytes(size_t n) { return (n + 127) / 128 * 128 * 64; }
+size_t fqk_x25519_scratch_bytes(size_t n) { return x25519_scratch_bytes(n); }
 cudaError_t fqk_x25519(const void* k, const void* u, void* out, size_t n, void* scratch, cudaStream_t s) {
   mock_stream_enqueue(s, [=] { memset(scratch, 0x11, fqk_x25519_scratch_bytes(n)); sim_x25519_batched((cu8)k, (cu8)u, (u8)out, n, 16); });
   return cudaSuccess;

@@ -1,7 +1,7 @@
-// prep_ab.cu -- developer experiment: k_dh_prep (and the whole three-kernel step) built from the product headers with whatever
-// -D switches are under test, timed alone on 2^20 rows.  Results are not checked here (tests/ does that); inputs are the
-// encodings of [k]G produced by the comb kernel, so every row is a valid point.
-//   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo [-D...] -o prep_ab prep_ab.cu ../../fourq_b200/csrc/kernels_comb.cu
+// prep_ab.cu -- developer experiment: k_dh_prep (and the whole three-kernel step) built from the product headers, as they
+// stand or edited for the variant under test, timed alone on 2^20 rows.  Results are not checked here (tests/ does that);
+// inputs are the encodings of [k]G produced by the comb kernel, so every row is a valid point.
+//   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -o prep_ab prep_ab.cu ../../fourq_b200/csrc/kernels_comb.cu
 #include <cstdio>
 #include <cstdlib>
 #include "../../fourq_b200/csrc/kernels_dh.cuh"
@@ -9,7 +9,6 @@
 
 cudaError_t fqk_comb_init(void** tabs_out, cudaStream_t s);
 cudaError_t fqk_comb(int dh, int strict, const void* tabs, const void* k, void* out, void* status, size_t n, void* scratch, int sms, cudaStream_t s);
-size_t fqk_comb_scratch_bytes(size_t n);
 
 int main(int argc, char** argv) {
   const size_t n = 1 << 20;

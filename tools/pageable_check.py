@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """End-to-end DH rate with page-locked vs ordinary (pageable) numpy arrays, in the combinations a caller can produce.
-    [FQ_TRACE=1] [FQ_COPY_THREADS=n] python tools/pageable_check.py"""
+    [FQ_TRACE=1] python tools/pageable_check.py"""
 import os, sys, time, numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import fourq_b200 as fq
