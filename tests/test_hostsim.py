@@ -319,6 +319,82 @@ def test_adversarial_grid_vs_c_oracle(sim):
         assert (st == wst).all() and (out == want).all(), fn
 
 
+def _sim_rows(sim, fn, k, pt, width):
+    n = len(k)
+    out = np.full((n, width), 0xEE, np.uint8); st = np.full(n, 0xEE, np.uint8)
+    assert getattr(sim, fn)(_p(k), _p(pt), _p(out), _p(st), ctypes.c_size_t(n)) == 0
+    return out, st
+
+
+def test_torsion_grid_vs_c_oracle(sim):
+    """tests/torsion.py: the 392 points of the 392-torsion subgroup and prime-order points shifted by each of them, through the
+    DEVICE DH code (both algorithms, encoded and affine entry points).  DH_core clears the cofactor first, so a pure torsion
+    point gives the neutral point (status 5; 3 where decode stops at the reference's t == 0 quirk, i.e. the points of order
+    1, 2 and 4) with a zero-filled row, and DH(k, P + T) == DH(k, P) for every T."""
+    import torsion
+    from oracle import c_oracle as C
+    for affine, (k, pt, same) in ((False, torsion.grid()), (True, torsion.affine_grid())):
+        want, wst = (C.dh_affine if affine else C.dh)(k, pt)
+        tors = same < 0
+        if affine:
+            assert (wst[tors] == 5).all()
+        else:
+            quirk = np.array([O.decode_status(bytes(e))[0] == O.ST_QUIRK_T0 for e in pt])
+            assert quirk.sum() == 4 * 3 and (quirk <= tors).all()                        # O, (0, -1), (+-i, 0), three scalars each
+            assert (wst[quirk] == 3).all() and (wst[tors & ~quirk] == 5).all()
+        assert not want[tors].any()
+        assert (wst[~tors] == 0).all() and (want[~tors] == want[same[~tors]]).all()
+        for fn in ("sim_dh_endo", "sim_dh") if not affine else ("sim_dh_endo_affine", "sim_dh_affine"):
+            out, st = _sim_rows(sim, fn, k, pt, 64 if affine else 32)
+            assert (st == wst).all() and (out == want).all(), fn
+
+
+def test_torsion_grid_vs_plain_group_law(sim):
+    """DH rows of the device code (simulation) against [392 k]A computed with the plain affine group law of tests/torsion.py,
+    which shares no formula or recoding with the oracle: 32 pure torsion rows and 32 shifted rows of each grid."""
+    import torsion
+    rng = random.Random(392)
+    for affine, (k, pt, same) in ((False, torsion.grid()), (True, torsion.affine_grid())):
+        tors = np.flatnonzero(same < 0)
+        rows = rng.sample(list(tors), 32) + rng.sample(list(np.flatnonzero(same >= 0)), 32)
+        for fn in ("sim_dh_endo", "sim_dh") if not affine else ("sim_dh_endo_affine", "sim_dh_affine"):
+            out, st = _sim_rows(sim, fn, k[rows], pt[rows], 64 if affine else 32)
+            for i, r in enumerate(rows):
+                if affine:
+                    ws, A = O.ST_OK, O.xy_from_bytes(pt[r])
+                else:
+                    ws, A = O.decode_status(bytes(pt[r]))
+                Q = torsion.dh_plain(int.from_bytes(bytes(k[r]), "little"), A) if ws == O.ST_OK else None
+                if ws == O.ST_OK:
+                    ws = O.ST_OK if Q is not None else O.ST_NEUTRAL
+                w = bytes(64 if affine else 32) if Q is None else (torsion.xy(Q) if affine else torsion.enc(Q))
+                assert (int(st[i]), bytes(out[i])) == (ws, w), (fn, r)
+                assert (Q is None) == (r in tors)
+
+
+def test_fixed_base_vs_plain_group_law(sim):
+    """[k]G (MUL_windowed, MUL_endo, per-digit comb) and [392 k]G with the neutral check (the DH_base variants) of the device
+    code against the plain affine group law of tests/torsion.py, on special and random scalars."""
+    import adversarial
+    import torsion
+    rng = random.Random(393)
+    ks = adversarial.special_scalars()
+    ks = rng.sample(ks, 40) + [0, O.N, 2 * O.N] + [rng.getrandbits(256) for _ in range(21)]
+    k = _rows([x.to_bytes(32, "little") for x in ks]).reshape(-1, 32)
+    G = (O.GX, O.GY)
+    want_mul = [torsion.enc(torsion.mul(x % O.N, G)) for x in ks]
+    want_dh = [(5, bytes(32)) if Q is None else (0, torsion.enc(Q)) for Q in (torsion.dh_plain(x, G) for x in ks)]
+    assert sum(w[0] == 5 for w in want_dh) == sum(x % O.N == 0 for x in ks) >= 3
+    n = len(ks)
+    for fn, mode in (("sim_fixed_base", 0), ("sim_fixed_base", 2), ("sim_comb", 0), ("sim_fixed_base", 1), ("sim_fixed_base", 3), ("sim_comb", 1)):
+        out = np.full((n, 32), 0xEE, np.uint8); st = np.full(n, 0xEE, np.uint8)
+        assert getattr(sim, fn)(mode, _p(k), _p(out), _p(st), ctypes.c_size_t(n)) == 0
+        if mode & 1:
+            assert [(int(s), bytes(o)) for s, o in zip(st, out)] == want_dh, (fn, mode)
+        else:
+            assert [bytes(o) for o in out] == want_mul, (fn, mode)
+
+
 def test_x25519_special_values_vs_oracle(sim):
     """The device X25519 code (simulation) on special u coordinates x special scalars and 200 random rows vs the oracle."""
     rng = random.Random(91)
@@ -381,8 +457,9 @@ def test_batched_inversion_with_zero_rows_in_every_position(sim, rows_per_thread
 
 
 def test_finish_kernel_mixed_groups(sim):
-    """batchinv.cuh FinishIO (k_dh_finish): projective rows with Z = 0 / failed status / the neutral point mixed with good rows in
-    one shared inversion; compared with the per-row R1toAffine + neutral check + encode of the oracle."""
+    """batchinv.cuh FinishIO (k_dh_finish): projective rows with Z = 0 (also as p in either half) / failed status / the neutral
+    point mixed with good rows in one shared inversion; compared with the per-row R1toAffine + neutral check + encode of the
+    oracle.  A zero Z that entered the shared product would zero the results of every row in its group."""
     rng = random.Random(41)
     p = O.P127
     G = (O.GX, O.GY)
@@ -404,12 +481,14 @@ def test_finish_kernel_mixed_groups(sim):
         elif r < 0.2:
             st = rng.choice([1, 2, 3, 4])                                                          # failed validation, harmless coordinates
         elif r < 0.3:
-            X, Y, Z = (0, 0), lam, lam                                                             # the neutral point (0, 1)
+            X, Y, Z = rng.choice([(0, 0), (p, 0), (p, p)]), lam, lam                              # the neutral point (0, 1), x = 0 in any form
+        elif r < 0.4:                                                                              # failed validation, Z a non-canonical zero:
+            Z, st = rng.choice([(p, 0), (0, p), (p, p)]), rng.choice([1, 2, 3, 4])                 # "zero is 0 or p" (fp.cuh fp_is_zero)
         rows.append(b"".join(v.to_bytes(16, "little") for v in (X[0], X[1], Y[0], Y[1], Z[0], Z[1])))
         st_in.append(st)
         if st != 0:
             want.append(bytes(32)); wst.append(st)
-        elif X == (0, 0) and Y == Z:
+        elif (X[0] % p, X[1] % p) == (0, 0) and Y == Z:
             want.append(bytes(32)); wst.append(5)
         else:
             zi = O.f2_inv(Z)
