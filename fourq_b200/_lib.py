@@ -58,6 +58,9 @@ def bind(L):
         "fq_dh_endo_base": ([vp, vp, vp, sz, i], i), "fq_mul_endo_base": ([vp, vp, sz, i], i),
         "fq_dh_base_comb": ([vp, vp, vp, sz, i], i), "fq_mul_base_comb": ([vp, vp, sz, i], i),
         "fq_x25519": ([vp, vp, vp, sz, i], i),
+        "fq_base_create": ([vp, i, vp, ctypes.POINTER(vp)], i), "fq_base_destroy": ([vp], i),
+        "fq_dh_fixed": ([vp, vp, vp, vp, sz, i], i), "fq_mul_fixed": ([vp, vp, vp, sz, i], i),
+        "fq_base_dev_run": ([vp, i, i, vp, vp, vp, sz, i, ctypes.POINTER(ctypes.c_float)], i),
         "fq_host_alloc": ([ctypes.POINTER(vp), sz], i), "fq_host_free": ([vp], i),
         "fq_host_alloc_sliced": ([ctypes.POINTER(vp), sz, sz, i], i), "fq_device_numa_node": ([i], i),
         "fq_dev_alloc": ([i, ctypes.POINTER(vp), sz], i), "fq_dev_free": ([i, vp], i),
@@ -76,7 +79,8 @@ def bind(L):
 EXPORTS = ["fq_version", "fq_device_count", "fq_last_error", "fq_set_device_base", "fq_set_select_mode", "fq_get_select_mode", "fq_trim", "fq_last_kernel_ms", "fq_last_rows_per_device", "fq_fp2_mul",
            "fq_fp2_sqr", "fq_fp2_inv", "fq_fp2_add", "fq_fp2_sub", "fq_fp2_neg", "fq_fp2_conj", "fq_fp2_invsqrt", "fq_fp_select", "fq_fp2_select", "fq_fp_op", "fq_fp25519_op", "fq_decode", "fq_decode_spec", "fq_encode", "fq_point_on_curve",
            "fq_dh", "fq_dh_affine", "fq_dh_base", "fq_mul_base", "fq_dh_endo", "fq_dh_endo_affine", "fq_dh_endo_base",
-           "fq_mul_endo_base", "fq_dh_base_comb", "fq_mul_base_comb", "fq_x25519", "fq_host_alloc", "fq_host_free", "fq_host_alloc_sliced", "fq_device_numa_node",
+           "fq_mul_endo_base", "fq_dh_base_comb", "fq_mul_base_comb", "fq_base_create", "fq_base_destroy", "fq_dh_fixed", "fq_mul_fixed",
+           "fq_base_dev_run", "fq_x25519", "fq_host_alloc", "fq_host_free", "fq_host_alloc_sliced", "fq_device_numa_node",
            "fq_dev_alloc", "fq_dev_free", "fq_dev_upload", "fq_dev_download", "fq_dev_run", "fq_dev_run3", "fq_dev_last_phase_ms", "fq_dev_flush_l2", "fq_imad_peak"]
 
 

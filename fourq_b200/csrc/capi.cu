@@ -40,6 +40,20 @@
 #endif
 #include "../../include/fourq_b200.h"
 #include "kernels.h"
+#ifdef FQ_MOCK_CUDA
+// The mock kernels of the host-engine tests that predate registered bases do not define the table build: a weak reference lets
+// those builds link, and base_tables reports the missing kernel (tests/hostsim/mock_kernels_fixed.cpp defines it).
+extern cudaError_t fqk_comb_build(const void* xy, void** tabs_out, cudaStream_t s) __attribute__((weak));
+#endif
+
+// A caller-registered base point (fq_base_create): its canonical affine coordinates and, per GPU, the device buffer of its
+// two per-digit tables (of P and of [392]P, kernels.h fqk_comb_build).  A GPU's tables are built by the first call that uses
+// the handle on that GPU, under that GPU's DevCtx::mu, and only read or freed under it; they are multiples of a public
+// point, so fq_trim keeps them.
+struct fq_base {
+  uint8_t xy[64];
+  mutable void* tabs[16] = {};        // one entry per device (kMaxDev)
+};
 
 namespace {
 
@@ -47,6 +61,10 @@ constexpr int kSlots = 4;                        // stream slots per GPU = chunk
 constexpr int kMaxDev = 16;
 constexpr int kOperands = 5;                      // a, b, c (inputs), out, status
 constexpr size_t kFlushBytes = 256u << 20;        // > 126 MB L2
+static_assert(sizeof(fq_base::tabs) / sizeof(void*) == kMaxDev, "one table pointer per device");
+// internal op codes (not FQ_DEVOP_*): fq_dh_fixed / fq_mul_fixed, k_comb on the tables of a registered base.  They only
+// run through run_host and dev_run with that base; fq_dev_run refuses them.
+constexpr int kOpDhFixed = 64, kOpMulFixed = 65;
 
 thread_local char tl_err[512] = "";
 thread_local float tl_kernel_ms = 0.f;
@@ -109,6 +127,8 @@ OpDesc describe(int op) {
     case FQ_DEVOP_MUL_BASE: case FQ_DEVOP_MUL_ENDO_BASE: return {op, {32, 0, 0}, 32, false, M / 8, SCRATCH_FIXED_BASE};
     case FQ_DEVOP_DH_BASE_COMB: return {op, {32, 0, 0}, 32, true, kCombChunkRows, SCRATCH_FIXED_BASE, 2};
     case FQ_DEVOP_MUL_BASE_COMB: return {op, {32, 0, 0}, 32, false, kCombChunkRows, SCRATCH_FIXED_BASE, 2};
+    case kOpDhFixed: return {op, {32, 0, 0}, 32, true, kCombChunkRows, SCRATCH_FIXED_BASE, 2};
+    case kOpMulFixed: return {op, {32, 0, 0}, 32, false, kCombChunkRows, SCRATCH_FIXED_BASE, 2};
     case FQ_DEVOP_X25519: return {op, {32, 32, 0}, 32, false, M / 8, SCRATCH_X25519};
     case FQ_DEVOP_F25519_BASE + FQ_FP_MUL: case FQ_DEVOP_F25519_BASE + FQ_FP_ADD: case FQ_DEVOP_F25519_BASE + FQ_FP_SUB: return {op, {32, 32, 0}, 32, false, M};
     case FQ_DEVOP_F25519_BASE + FQ_FP_SQR: return {op, {32, 0, 0}, 32, false, M};
@@ -327,6 +347,15 @@ int device_count() {
   return n > kMaxDev ? kMaxDev : n;
 }
 
+// caller holds c.mu and the device is current: the tables of base b on this GPU exist (built here on first use)
+int base_tables(DevCtx& c, const fq_base& b) {
+#ifdef FQ_MOCK_CUDA
+  if (!fqk_comb_build) return fail(FQ_ERR_CUDA, "this mock build has no table-build kernel");
+#endif
+  if (!b.tabs[c.dev]) CU(fqk_comb_build(b.xy, &b.tabs[c.dev], c.slot[0].st));
+  return FQ_OK;
+}
+
 // caller holds c.mu
 int ctx_init(DevCtx& c) {
   CU(cudaSetDevice(c.dev));
@@ -409,11 +438,14 @@ PtrKind classify(const void* p, size_t bytes) {
 
 // ---------------------------------------------------------------- kernels of one chunk
 
-cudaError_t launch(const DevCtx& cx, int op, const void* a, const void* b, const void* c, void* out, void* status, size_t n, cudaStream_t s, void* scratch, cudaEvent_t* ev = nullptr) {
+// tabs: the tables of the registered base on this GPU (kOpDhFixed, kOpMulFixed), else unused
+cudaError_t launch(const DevCtx& cx, int op, const void* tabs, const void* a, const void* b, const void* c, void* out, void* status, size_t n, cudaStream_t s, void* scratch, cudaEvent_t* ev = nullptr) {
   const int strict = strict_mode();
   switch (op) {
     case FQ_DEVOP_DH_BASE_COMB: return fqk_comb(1, strict, cx.comb, a, out, status, n, scratch, cx.sms, s);
     case FQ_DEVOP_MUL_BASE_COMB: return fqk_comb(0, strict, cx.comb, a, out, nullptr, n, scratch, cx.sms, s);
+    case kOpDhFixed: return fqk_comb(1, strict, tabs, a, out, status, n, scratch, cx.sms, s);
+    case kOpMulFixed: return fqk_comb(0, strict, tabs, a, out, nullptr, n, scratch, cx.sms, s);
     case FQ_DEVOP_FP2_MUL: return fqk_fp2_op(FQK_MUL, a, b, out, n, s);
     case FQ_DEVOP_FP2_SQR: return fqk_fp2_op(FQK_SQR, a, b, out, n, s);
     case FQ_DEVOP_FP2_INV: return fqk_fp2_op(FQK_INV, a, b, out, n, s);
@@ -455,6 +487,7 @@ struct SliceJob {
   OpDesc d;
   const uint8_t* in[3] = {nullptr, nullptr, nullptr};      // whole-call buffers
   uint8_t* out = nullptr; uint8_t* status = nullptr;
+  const fq_base* base = nullptr;                           // the registered base of kOpDhFixed / kOpMulFixed
   CallWork* work = nullptr; int index = 0;                 // the call's rows and this GPU's slice number
   size_t rows_done = 0;
   bool grew = false;                                       // buffers were allocated during this job: its speed is not representative
@@ -509,7 +542,7 @@ int feed_slice(DevCtx& c, SliceJob* j) {
       const double te0 = now_ms();
       if (ci == 0) CU(cudaEventRecord(c.job_e0, s.st));
       CU(cudaEventRecord(s.e0, s.st));
-      CU(launch(c, d.op, s.dbuf[0], s.dbuf[1], s.dbuf[2], s.dbuf[3], s.dbuf[4], rows, s.st, s.scratch));
+      CU(launch(c, d.op, j->base ? j->base->tabs[c.dev] : nullptr, s.dbuf[0], s.dbuf[1], s.dbuf[2], s.dbuf[3], s.dbuf[4], rows, s.st, s.scratch));
       CU(cudaEventRecord(s.e1, s.st));
       CU(cudaMemcpyAsync(j->pinned[3] ? (void*)(j->out + r0 * d.out_bytes) : s.hbuf[3], s.dbuf[3], rows * d.out_bytes, cudaMemcpyDeviceToHost, s.st));
       if (d.status) CU(cudaMemcpyAsync(j->pinned[4] ? (void*)(j->status + r0) : s.hbuf[4], s.dbuf[4], rows, cudaMemcpyDeviceToHost, s.st));
@@ -574,6 +607,7 @@ void feeder_main(DevCtx* cp) {
     {
       std::lock_guard<std::mutex> dl(c.mu);
       int rc = ctx_init(c);
+      if (rc == FQ_OK && j->base) rc = base_tables(c, *j->base);
       if (rc != FQ_OK) job_fail(c, j, rc); else feed_slice(c, j);
     }
     CallState* cs = j->call;
@@ -592,7 +626,7 @@ void submit(DevCtx& c, SliceJob* j) {
   c.qcv.notify_one();
 }
 
-int run_host(int op, const uint8_t* a, const uint8_t* b, const uint8_t* cbuf, uint8_t* out, uint8_t* status, size_t n, int ndev) {
+int run_host(int op, const uint8_t* a, const uint8_t* b, const uint8_t* cbuf, uint8_t* out, uint8_t* status, size_t n, int ndev, const fq_base* fb = nullptr) {
   tl_kernel_ms = 0.f;
   const OpDesc d = describe(op);
   if (d.op < 0) return fail(FQ_ERR_ARG, "unknown operation %d", op);
@@ -630,7 +664,7 @@ int run_host(int op, const uint8_t* a, const uint8_t* b, const uint8_t* cbuf, ui
   for (int i = 0; i < ndev; i++) {
     if (work.r[(size_t)i].lo >= work.r[(size_t)i].hi) break;          // fewer rows than GPUs: the empty slices get no job
     SliceJob& j = jobs[(size_t)i];
-    j.d = dj; j.in[0] = a; j.in[1] = b; j.in[2] = cbuf; j.out = out; j.status = status;
+    j.d = dj; j.in[0] = a; j.in[1] = b; j.in[2] = cbuf; j.out = out; j.status = status; j.base = fb;
     j.work = &work; j.index = i;
     for (int w = 0; w < kOperands; w++) j.pinned[w] = pinned[w];
     j.call = &cs;
@@ -721,6 +755,32 @@ struct DevLock {
   ~DevLock() { if (c) c->mu.unlock(); }
 };
 
+// fq_dev_run3 on GPU `dev`, with the tables of `base` for kOpDhFixed / kOpMulFixed
+int dev_run(const fq_base* base, int op, int dev, const void* a, const void* b, const void* c, void* out, void* status, size_t n, int iters, float* ms) {
+  DevLock L(dev); if (L.rc != FQ_OK) return L.rc;
+  const OpDesc d = describe(op);
+  if (d.op < 0 || iters < 1) return fail(FQ_ERR_ARG, "bad op/iters");
+  if ((op == FQ_DEVOP_FP2_INV || op == FQ_DEVOP_F25519_BASE + FQ_FP_INV) && a == out) return fail(FQ_ERR_ARG, "inv: out must not alias a (the prefix products are parked in out)");
+  DevCtx& cx = *L.c;
+  Slot& s = cx.slot[0];
+  int rc;
+  if (base && (rc = base_tables(cx, *base)) != FQ_OK) return rc;
+  if ((rc = scratch_reserve(s, d.scratch, n)) != FQ_OK) return rc;
+  cudaEvent_t ph[4];
+  for (int i = 0; i < 4; i++) CU(cudaEventCreate(&ph[i]));
+  CU(cudaEventRecord(s.e0, s.st));
+  for (int i = 0; i < iters; i++) CU(launch(cx, op, base ? base->tabs[dev] : nullptr, a, b, c, out, status, n, s.st, s.scratch, (d.var_dh && i == iters - 1) ? ph : nullptr));
+  CU(cudaEventRecord(s.e1, s.st));
+  CU(cudaEventSynchronize(s.e1));
+  float t = 0.f;
+  CU(cudaEventElapsedTime(&t, s.e0, s.e1));
+  tl_phase_ms[0] = tl_phase_ms[1] = tl_phase_ms[2] = 0.f;
+  if (d.var_dh && n > 0) for (int i = 0; i < 3; i++) CU(cudaEventElapsedTime(&tl_phase_ms[i], ph[i], ph[i + 1]));
+  for (int i = 0; i < 4; i++) cudaEventDestroy(ph[i]);
+  if (ms) *ms = t / iters;
+  return FQ_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -794,6 +854,57 @@ int fq_mul_endo_base(const uint8_t* k, uint8_t* enc_out, size_t n, int ndev) { r
 int fq_dh_base_comb(const uint8_t* k, uint8_t* enc_out, uint8_t* status, size_t n, int ndev) { return run_host(FQ_DEVOP_DH_BASE_COMB, k, nullptr, nullptr, enc_out, status, n, ndev); }
 int fq_mul_base_comb(const uint8_t* k, uint8_t* enc_out, size_t n, int ndev) { return run_host(FQ_DEVOP_MUL_BASE_COMB, k, nullptr, nullptr, enc_out, nullptr, n, ndev); }
 int fq_x25519(const uint8_t* k, const uint8_t* u, uint8_t* out, size_t n, int ndev) { return run_host(FQ_DEVOP_X25519, k, u, nullptr, out, nullptr, n, ndev); }
+
+// Validation runs on the GPU through the kernels of fq_decode, or of fq_fp2_add (x + 0 and y + 0: each half reduced mod p, as
+// the affine DH entry points read a point) and fq_point_on_curve, one row each.
+int fq_base_create(const uint8_t* pt, int affine, uint8_t* status, fq_base** out) {
+  if (!pt || !status || !out) return fail(FQ_ERR_ARG, "null pointer");
+  *out = nullptr;
+  uint8_t xy[64], st = FQ_ST_OK;
+  int rc;
+  if (affine) {
+    static const uint8_t zero[64] = {0};
+    uint8_t ok = 0;
+    if ((rc = run_host(FQ_DEVOP_FP2_ADD, pt, zero, nullptr, xy, nullptr, 2, 1)) != FQ_OK) return rc;
+    if ((rc = run_host(FQ_DEVOP_ON_CURVE, xy, nullptr, nullptr, &ok, nullptr, 1, 1)) != FQ_OK) return rc;
+    if (!ok) st = FQ_ST_NOT_ON_CURVE;
+  } else if ((rc = run_host(FQ_DEVOP_DECODE, pt, nullptr, nullptr, xy, &st, 1, 1)) != FQ_OK) {
+    return rc;
+  }
+  *status = st;
+  if (st != FQ_ST_OK) return FQ_OK;
+  fq_base* b = new fq_base;
+  memcpy(b->xy, xy, sizeof(xy));
+  *out = b;
+  return FQ_OK;
+}
+int fq_base_destroy(fq_base* base) {
+  if (!base) return FQ_OK;
+  int rc = FQ_OK;
+  for (int dev = 0; dev < kMaxDev; dev++) {
+    DevCtx& c = ctx_of(dev);
+    std::lock_guard<std::mutex> l(c.mu);
+    if (!base->tabs[dev]) continue;
+    cudaError_t e = cudaSetDevice(dev);
+    if (e == cudaSuccess) e = cudaFree(base->tabs[dev]);
+    if (e != cudaSuccess && rc == FQ_OK) rc = fail(FQ_ERR_CUDA, "freeing the tables of a base on device %d failed: %s", dev, cudaGetErrorString(e));
+    base->tabs[dev] = nullptr;
+  }
+  delete base;
+  return rc;
+}
+int fq_dh_fixed(const fq_base* base, const uint8_t* k, uint8_t* enc_out, uint8_t* status, size_t n, int ndev) {
+  if (!base) return fail(FQ_ERR_ARG, "null base");
+  return run_host(kOpDhFixed, k, nullptr, nullptr, enc_out, status, n, ndev, base);
+}
+int fq_mul_fixed(const fq_base* base, const uint8_t* k, uint8_t* enc_out, size_t n, int ndev) {
+  if (!base) return fail(FQ_ERR_ARG, "null base");
+  return run_host(kOpMulFixed, k, nullptr, nullptr, enc_out, nullptr, n, ndev, base);
+}
+int fq_base_dev_run(const fq_base* base, int dh, int dev, const void* k, void* out, void* status, size_t n, int iters, float* ms) {
+  if (!base) return fail(FQ_ERR_ARG, "null base");
+  return dev_run(base, dh ? kOpDhFixed : kOpMulFixed, dev, k, nullptr, nullptr, out, dh ? status : nullptr, n, iters, ms);
+}
 
 int fq_host_alloc(void** p, size_t bytes) {
   if (!p) return fail(FQ_ERR_ARG, "null pointer");
@@ -871,27 +982,8 @@ int fq_dev_download(int dev, void* dst, const void* src, size_t bytes) {
   return FQ_OK;
 }
 int fq_dev_run3(int op, int dev, const void* a, const void* b, const void* c, void* out, void* status, size_t n, int iters, float* ms) {
-  DevLock L(dev); if (L.rc != FQ_OK) return L.rc;
-  const OpDesc d = describe(op);
-  if (d.op < 0 || iters < 1) return fail(FQ_ERR_ARG, "bad op/iters");
-  if ((op == FQ_DEVOP_FP2_INV || op == FQ_DEVOP_F25519_BASE + FQ_FP_INV) && a == out) return fail(FQ_ERR_ARG, "inv: out must not alias a (the prefix products are parked in out)");
-  DevCtx& cx = *L.c;
-  Slot& s = cx.slot[0];
-  int rc;
-  if ((rc = scratch_reserve(s, d.scratch, n)) != FQ_OK) return rc;
-  cudaEvent_t ph[4];
-  for (int i = 0; i < 4; i++) CU(cudaEventCreate(&ph[i]));
-  CU(cudaEventRecord(s.e0, s.st));
-  for (int i = 0; i < iters; i++) CU(launch(cx, op, a, b, c, out, status, n, s.st, s.scratch, (d.var_dh && i == iters - 1) ? ph : nullptr));
-  CU(cudaEventRecord(s.e1, s.st));
-  CU(cudaEventSynchronize(s.e1));
-  float t = 0.f;
-  CU(cudaEventElapsedTime(&t, s.e0, s.e1));
-  tl_phase_ms[0] = tl_phase_ms[1] = tl_phase_ms[2] = 0.f;
-  if (d.var_dh && n > 0) for (int i = 0; i < 3; i++) CU(cudaEventElapsedTime(&tl_phase_ms[i], ph[i], ph[i + 1]));
-  for (int i = 0; i < 4; i++) cudaEventDestroy(ph[i]);
-  if (ms) *ms = t / iters;
-  return FQ_OK;
+  if (op == kOpDhFixed || op == kOpMulFixed) return fail(FQ_ERR_ARG, "bad op/iters");      // need a base: fq_base_dev_run
+  return dev_run(nullptr, op, dev, a, b, c, out, status, n, iters, ms);
 }
 int fq_dev_run(int op, int dev, const void* a, const void* b, void* out, void* status, size_t n, int iters, float* ms) {
   return fq_dev_run3(op, dev, a, b, nullptr, out, status, n, iters, ms);

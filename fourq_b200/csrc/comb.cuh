@@ -81,11 +81,17 @@ template <bool STRICT = FQ_STRICT_DEFAULT> FQ_FN ptR1 mul_comb(const scal& k, co
   return Q;
 }
 
-// Table construction, one call per (base, digit): out = the 192 words of T_i for B = G (which = 0) or [392]G (which = 1).
+// The base whose tables give MUL (dh = 0: B = P, curve4q.py:582-584) or DH (dh = 1: B = [392]P, curve4q.py:450-460) of the
+// point P = (x, y).  The tables of G built at context creation and those of a caller-registered point both start here.
+FQ_FN ptR1 comb_base(int dh, const fp2& x, const fp2& y) { return dh ? pt_clear_cofactor(x, y) : pt_from_affine(x, y); }
+
+// Table construction, one call per (base, digit): out = the 192 words of T_i for the base B (comb_base).
 // P = [16^i]B by 4 i doublings, then the odd multiples as in table_windowed (curve4q.py:179-185), each normalised to
-// affine.  Run once per device at context creation (126 threads); also by the CPU simulation in tests/hostsim.
-FQ_FN void comb_build_digit(int which, int i, u32* out) {
-  ptR1 P = (which == 0) ? pt_from_affine(curve_gx(), curve_gy()) : pt_clear_cofactor(curve_gx(), curve_gy());
+// affine.  Every entry is canonical affine, so the words depend only on the group element B, not on its coordinates.
+// Run once per device at context creation for G (k_comb_build, 126 threads), once per device for a registered point, and
+// by the CPU simulation in tests/hostsim.
+FQ_FN void comb_build_digit(const ptR1& B, int i, u32* out) {
+  ptR1 P = B;
   FQ_NOUNROLL
   for (int t = 0; t < 4 * i; t++) pt_dbl_c(&P);
   ptR1 P2 = P;
@@ -106,3 +112,5 @@ FQ_FN void comb_build_digit(int which, int i, u32* out) {
     if (j < 7) { ptR2 Mr2; pt_r1_to_r2_c(&Mr2, &M); pt_add_core_c(&M, &P23, &Mr2); }     // M += 2P
   }
 }
+// the same for the tables of G (which = 0) and [392]G (which = 1), as the CPU simulation of tests/hostsim builds them
+FQ_FN void comb_build_digit(int which, int i, u32* out) { comb_build_digit(comb_base(which, curve_gx(), curve_gy()), i, out); }

@@ -52,8 +52,11 @@ cudaError_t fqk_dh_endo_init();
 cudaError_t fqk_dh_windowed(int affine, int strict, const void* k, const void* pt, void* out, void* status, size_t n, void* scratch, cudaStream_t s, cudaEvent_t* ev);
 cudaError_t fqk_dh_endo(int affine, int strict, const void* k, const void* pt, void* out, void* status, size_t n, void* scratch, cudaStream_t s, cudaEvent_t* ev);
 cudaError_t fqk_fixed_base(int dh, int endo, int strict, const void* k, void* out, void* status, size_t n, void* scratch, cudaStream_t s);   // scratch: fqk_comb_scratch_bytes(n)
-// fixed-base per-digit tables (kernels_comb.cu): tabs is the device buffer returned by fqk_comb_init
+// fixed-base per-digit tables (kernels_comb.cu): tabs is a device buffer of [2][FQ_COMB_WORDS] words, the tables of P
+// (fqk_comb with dh = 0) and of [392]P (dh = 1), returned by fqk_comb_init (P = G) or fqk_comb_build (P = the canonical affine
+// point xy, 64 host bytes).  Both synchronise the stream and free the buffer on every error path; the caller frees it with cudaFree.
 cudaError_t fqk_comb_init(void** tabs_out, cudaStream_t s);
+cudaError_t fqk_comb_build(const void* xy, void** tabs_out, cudaStream_t s);
 cudaError_t fqk_comb(int dh, int strict, const void* tabs, const void* k, void* out, void* status, size_t n, void* scratch, int sms, cudaStream_t s);   // scratch: fqk_comb_scratch_bytes(n)
 cudaError_t fqk_x25519(const void* k, const void* u, void* out, size_t n, void* scratch, cudaStream_t s);   // scratch: fqk_x25519_scratch_bytes(n)
 cudaError_t fqk_f25_op(int op, const void* a, const void* b, void* out, size_t n, cudaStream_t s);   // GF(2^255-19), 32-byte rows, op = FQ_FP_MUL.._SUB of the header

@@ -10,6 +10,8 @@
     y of DH_*(m, decode(B))  (draft :707-714)       DH(k, B, y_only=True) -> (y[N,32], status[N])
     DH_*(m, G, table=T392)             :743-762     DH_base(k[N,32], algorithm=) -> (B[N,32], status[N])
     MUL_*(m, G, table=T) -> [m]G       :582-584     MUL_base(k[N,32], algorithm=) -> B[N,32]
+    encode(DH_windowed(m, P)), one P                FixedBase(P).DH(k[N,32]) -> (B[N,32], status[N])
+    encode(MUL_windowed(m, P)), one P  :188-235     FixedBase(P).MUL(k[N,32]) -> B[N,32]
 
 algorithm = "windowed" runs MUL_windowed (curve4q.py:188-235), "endo" runs MUL_endo (curve4q.py:405-442); the results
 are bit-identical (the reference asserts it, curve4q.py:706-762), "endo" needs about 1.8x fewer field multiplications
@@ -21,6 +23,8 @@ Scalars are 32-byte little-endian unsigned rows (no clamping).  Exceptions of th
 failed rows are zero-filled.  `strict=True` raises the reference's message for the first failing row instead.
 decode() does not modify its argument (the reference clears bits in place, curve4q.py:56).
 """
+import ctypes
+
 import numpy as np
 
 from . import _lib
@@ -160,6 +164,80 @@ def MUL_base(k, ndev=1, out=None, algorithm=None):
     fn = getattr(_lib.lib(), {"windowed": "fq_mul_base", "endo": "fq_mul_endo_base", "comb": "fq_mul_base_comb"}[_alg(algorithm, base=True)])
     _lib.check(fn(_lib.ptr(k), _lib.ptr(out), k.shape[0], ndev))
     return out
+
+
+class FixedBase:
+    """One public point P registered for many scalars: fixed-base DH and scalar multiplication on per-digit tables of P and
+    [392]P, the comb of DH_base / MUL_base (algorithm="comb") for a point of the caller's choosing.
+
+    P is a 32-byte encoding, or with affine=True 64-byte x | y (each half reduced mod p).  It is validated once, as DH
+    validates it; an invalid P raises the reference's exception (STATUS_MESSAGES; AttributeError for the t == 0 quirk).
+    Each GPU builds the tables (2 x 48,384 B) on the first call that uses them there.
+
+    .DH(k)  per row, exactly DH(k, B) with B = P broadcast (encode(DH_windowed(k, P)) for an affine P): status 0 or 5.
+    .MUL(k) per row, encode(R1toAffine(MUL_windowed(k, P))) (curve4q.py:188-235) = encode([r]P) with r = k mod N, plus N if
+            that is even.  For P in the prime-order subgroup that is [k]P, and FixedBase(G).MUL(k) == MUL_base(k).  For a P
+            with a small-order component it is NOT [k]P, nor what MUL_endo gives: r and k differ by a multiple of N, which
+            does not annihilate the small-order part.
+
+    close() (or the end of a `with` block, or garbage collection) frees the tables; it must not run while a call that uses
+    the handle is in flight on another thread."""
+
+    def __init__(self, P, affine=False):
+        self.handle = None
+        width = 64 if affine else 32
+        if isinstance(P, (bytes, bytearray)):
+            P = np.frombuffer(bytes(P), np.uint8)
+        if not isinstance(P, np.ndarray) or P.dtype != np.uint8 or P.size != width:
+            raise ValueError("P must be %d bytes (a bytes object or a uint8 array)" % width)
+        P = np.ascontiguousarray(P).reshape(width)
+        st = np.zeros(1, np.uint8)
+        h = ctypes.c_void_p()
+        _lib.check(_lib.lib().fq_base_create(_lib.ptr(P), 1 if affine else 0, _lib.ptr(st), ctypes.byref(h)))
+        if st[0]:
+            raise (AttributeError if st[0] == ST_QUIRK_T0 else Exception)(STATUS_MESSAGES[int(st[0])])
+        self.handle = h
+
+    def _h(self):
+        if self.handle is None:
+            raise ValueError("FixedBase is closed")
+        return self.handle
+
+    def DH(self, k, ndev=1, strict=False, out=None, status=None, y_only=False):
+        """As DH(k, B, algorithm=any) with B = P on every row; y_only and strict as there."""
+        k = _lib.rows(k, 32, "k")
+        n = k.shape[0]
+        out = _buf(out, (n, 32), "out")
+        status = _buf(status, (n,), "status")
+        _lib.check(_lib.lib().fq_dh_fixed(self._h(), _lib.ptr(k), _lib.ptr(out), _lib.ptr(status), n, ndev))
+        if y_only:
+            out[:, 31] &= 0x7F
+        if strict:
+            _raise_first(status)
+        return out, status
+
+    def MUL(self, k, ndev=1, out=None):
+        k = _lib.rows(k, 32, "k")
+        out = _buf(out, (k.shape[0], 32), "out")
+        _lib.check(_lib.lib().fq_mul_fixed(self._h(), _lib.ptr(k), _lib.ptr(out), k.shape[0], ndev))
+        return out
+
+    def close(self):
+        if self.handle is not None:
+            h, self.handle = self.handle, None
+            _lib.check(_lib.lib().fq_base_destroy(h))
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:  # interpreter shutdown
+            pass
 
 
 def pack_affine(points):

@@ -125,6 +125,16 @@ def dev_run(op, dev, a, b, out, status, n, iters=1, c=None):
     return float(ms.value)
 
 
+def dev_run_fixed(base, dh, dev, k, out, status, n, iters=1):
+    """fq_dh_fixed (dh=True) or fq_mul_fixed (dh=False) of a curve4q.FixedBase on device buffers; returns average milliseconds
+    per launch.  The first call on a device builds the base's tables there, before the timed launches.  status may be None
+    for dh=False."""
+    ms = ctypes.c_float()
+    g = lambda x: x.ptr if x is not None else None  # noqa: E731
+    _lib.check(_lib.lib().fq_base_dev_run(base.handle, 1 if dh else 0, int(dev), g(k), g(out), g(status), int(n), int(iters), ctypes.byref(ms)))
+    return float(ms.value)
+
+
 def last_phase_ms():
     """CUDA-event milliseconds of the (prepare, ladder, finish) kernels of the last launch of the last DH dev_run."""
     ms = (ctypes.c_float * 3)()

@@ -153,6 +153,30 @@ FQ_API int fq_mul_endo_base(const uint8_t* k, uint8_t* enc_out, size_t n, int nd
 FQ_API int fq_mul_base_comb(const uint8_t* k, uint8_t* enc_out, size_t n, int ndev);
 FQ_API int fq_dh_base_comb(const uint8_t* k, uint8_t* enc_out, uint8_t* status, size_t n, int ndev);
 
+/* ---- Fixed base for a point the caller registers: one public point, many scalars, on per-digit tables as above.
+ * fq_base_create:  validates P once, exactly as the DH entry points do, on the GPU (one row):
+ *                  affine = 0: pt is a 32-byte encoding, *status = that of fq_decode (1-4, including 3 at the reference's
+ *                  t == 0 quirk, curve4q.py:49-96); affine = 1: pt is 64-byte x | y, each half reduced mod p, *status = 4
+ *                  if P is not on the curve (curve4q.py:447-448).
+ *                  Valid P: *status = 0 and *out = a new handle.  Invalid P: returns FQ_OK with *status != 0 and *out = NULL.
+ *                  A pure-torsion P is valid: fq_dh_fixed then gives status 5 on every row, as fq_dh does.
+ *                  Each GPU builds the tables of P and [392]P (2 x 48,384 B) on the first call that uses the handle there.
+ * fq_dh_fixed:     per row, exactly fq_dh(k, enc(P)) for an encoded registration, and encode(DH_windowed(k, P)) for an affine
+ *                  one (the bytes of fq_encode(fq_dh_affine(k, P))): DH_core (curve4q.py:446-462) computes Q = [392]P and
+ *                  MUL_windowed(m, Q) = [r]Q with r = m mod N, plus N if that is even (curve4q.py:216-219).  Status 0 or 5.
+ * fq_mul_fixed:    per row, encode(R1toAffine(MUL_windowed(k, P))) (curve4q.py:188-235) = encode([r]P) with the same r; no
+ *                  status, k = 0 mod N gives the encoding of the neutral point.  For a P with a small-order component this is
+ *                  NOT [k]P (r differs from k by a multiple of N, which does not kill the torsion part) and not what
+ *                  MUL_endo would give; for P in the prime-order subgroup it is [k]P, and a handle of G gives fq_mul_base.
+ * fq_base_destroy: frees the handle and its tables on every GPU (NULL is a no-op).  The handle must not be in use by a call
+ *                  in flight on any thread.  fq_trim keeps the tables (multiples of a public point).
+ * A handle may be used by several threads at once, on the same or on different GPUs. */
+typedef struct fq_base fq_base;
+FQ_API int fq_base_create(const uint8_t* pt, int affine, uint8_t* status, fq_base** out);
+FQ_API int fq_base_destroy(fq_base* base);
+FQ_API int fq_dh_fixed(const fq_base* base, const uint8_t* k, uint8_t* enc_out, uint8_t* status, size_t n, int ndev);
+FQ_API int fq_mul_fixed(const fq_base* base, const uint8_t* k, uint8_t* enc_out, size_t n, int ndev);
+
 /* ---- X25519 (RFC 7748): impl/curve25519.py:88-91 x25519(k, u) -> 32 bytes; k, u, out are (n,32) */
 FQ_API int fq_x25519(const uint8_t* k, const uint8_t* u, uint8_t* out, size_t n, int ndev);
 
@@ -210,6 +234,9 @@ FQ_API int fq_dev_run3(int op, int dev, const void* a, const void* b, const void
 /* CUDA-event milliseconds of the three kernels (prepare, ladder, finish) of the last launch of the last fq_dev_run of
  * this thread with a variable-base DH op (FQ_DEVOP_DH, _DH_AFFINE, _DH_ENDO, _DH_ENDO_AFFINE); zeros otherwise. */
 FQ_API int fq_dev_last_phase_ms(float* ms3);
+/* fq_dh_fixed (dh = 1) or fq_mul_fixed (dh = 0) on device buffers of GPU `dev`, `iters` launches as fq_dev_run (the first
+ * call on a GPU builds the base's tables there before timing); status may be NULL for dh = 0 */
+FQ_API int fq_base_dev_run(const fq_base* base, int dh, int dev, const void* k, void* out, void* status, size_t n, int iters, float* ms);
 /* writes `bytes` of zeros over a scratch buffer larger than L2 (used between timed iterations) */
 FQ_API int fq_dev_flush_l2(int dev);
 
