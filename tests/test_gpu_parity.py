@@ -476,6 +476,7 @@ def test_concurrent_callers_and_trim(fq):
     pub = fq.MUL_base(k)
     want_dh = fq.DH(k, pub)
     want_mul = fq.MUL_base(k, algorithm="endo")
+    want_x = fq.x25519(k, pub)
     res = {}
 
     def worker(name, fn):
@@ -489,6 +490,7 @@ def test_concurrent_callers_and_trim(fq):
     for t in ts:
         t.join()
     assert (res["dh"][0] == want_dh[0]).all() and (res["dh"][1] == want_dh[1]).all() and (res["mul"] == want_mul).all()
+    assert (res["x"] == want_x).all()
     fq.trim()
     again = fq.DH(k, pub)
     assert (again[0] == want_dh[0]).all() and (fq.MUL_base(k) == pub).all()
