@@ -27,6 +27,29 @@ namespace fqsim { extern thread_local u32 cc; }
 #define FQ_NOUNROLL _Pragma("unroll 1")
 #endif
 
+// Carry tracing (tests/hostsim/carry_trace.cpp, host simulation only, C++20): with FQ_HOSTSIM_CARRY every carry primitive takes
+// its call site as a defaulted argument and reports to fqsim::carry_event.  start ops (add_cc, sub_cc, mad_lo_cc) write the carry,
+// middle ops (addc_cc, subc_cc, madc_lo_cc, madc_hi_cc) read and write it, end ops (addc, subc, madc_hi) read it.
+#ifdef FQ_HOSTSIM_CARRY
+#ifndef FQ_HOSTSIM
+#error "FQ_HOSTSIM_CARRY is a variant of the host simulation (FQ_HOSTSIM)"
+#endif
+#include <source_location>
+namespace fqsim {
+enum CarryKind { CK_ADD_CC, CK_SUB_CC, CK_MAD_LO_CC, CK_ADDC_CC, CK_SUBC_CC, CK_MADC_LO_CC, CK_MADC_HI_CC, CK_ADDC, CK_SUBC, CK_MADC_HI };
+// exact0 = the op's exact result before its carry-in (mod 2^64: a subtraction wraps), cin = the carry flag (0 for a start op).
+// Returns the carry-in the op uses: cin, unless the tracer forces this site.  Carry-out and the 33-bit result follow from both.
+u32 carry_event(CarryKind kind, u32 cin, u64 exact0, const std::source_location& site);
+}
+#define FQ_SITE , const std::source_location fq_site = std::source_location::current()
+#define FQ_START(kind, exact0) ((void)fqsim::carry_event(fqsim::kind, 0, exact0, fq_site))
+#define FQ_CIN(kind, exact0) fqsim::carry_event(fqsim::kind, FQ_CC, exact0, fq_site)
+#else
+#define FQ_SITE
+#define FQ_START(kind, exact0) ((void)0)
+#define FQ_CIN(kind, exact0) FQ_CC
+#endif
+
 #ifdef FQ_HOSTSIM
 struct uint4 { u32 x, y, z, w; };
 FQ_FN uint4 make_uint4(u32 x, u32 y, u32 z, u32 w) { uint4 r = {x, y, z, w}; return r; }
@@ -43,44 +66,44 @@ FQ_FN uint4 make_uint4(u32 x, u32 y, u32 z, u32 w) { uint4 r = {x, y, z, w}; ret
 #endif
 
 // ---------------------------------------------------------------- add / sub with carry
-FQ_FN u32 add_cc(u32 a, u32 b) {
+FQ_FN u32 add_cc(u32 a, u32 b FQ_SITE) {
 #ifdef FQ_HOSTSIM
-  u64 s = (u64)a + b; FQ_CC = (u32)(s >> 32); return (u32)s;
+  u64 s = (u64)a + b; FQ_START(CK_ADD_CC, s); FQ_CC = (u32)(s >> 32); return (u32)s;
 #else
   u32 r; asm volatile("add.cc.u32 %0, %1, %2;" : "=r"(r) : "r"(a), "r"(b)); return r;
 #endif
 }
-FQ_FN u32 addc_cc(u32 a, u32 b) {
+FQ_FN u32 addc_cc(u32 a, u32 b FQ_SITE) {
 #ifdef FQ_HOSTSIM
-  u64 s = (u64)a + b + FQ_CC; FQ_CC = (u32)(s >> 32); return (u32)s;
+  u64 s = (u64)a + b + FQ_CIN(CK_ADDC_CC, (u64)a + b); FQ_CC = (u32)(s >> 32); return (u32)s;
 #else
   u32 r; asm volatile("addc.cc.u32 %0, %1, %2;" : "=r"(r) : "r"(a), "r"(b)); return r;
 #endif
 }
-FQ_FN u32 addc(u32 a, u32 b) {
+FQ_FN u32 addc(u32 a, u32 b FQ_SITE) {
 #ifdef FQ_HOSTSIM
-  return a + b + FQ_CC;
+  return a + b + FQ_CIN(CK_ADDC, (u64)a + b);
 #else
   u32 r; asm volatile("addc.u32 %0, %1, %2;" : "=r"(r) : "r"(a), "r"(b)); return r;
 #endif
 }
-FQ_FN u32 sub_cc(u32 a, u32 b) {
+FQ_FN u32 sub_cc(u32 a, u32 b FQ_SITE) {
 #ifdef FQ_HOSTSIM
-  u64 s = (u64)a - b; FQ_CC = (u32)(s >> 32) & 1; return (u32)s;   // CC = borrow
+  u64 s = (u64)a - b; FQ_START(CK_SUB_CC, s); FQ_CC = (u32)(s >> 32) & 1; return (u32)s;   // CC = borrow
 #else
   u32 r; asm volatile("sub.cc.u32 %0, %1, %2;" : "=r"(r) : "r"(a), "r"(b)); return r;
 #endif
 }
-FQ_FN u32 subc_cc(u32 a, u32 b) {
+FQ_FN u32 subc_cc(u32 a, u32 b FQ_SITE) {
 #ifdef FQ_HOSTSIM
-  u64 s = (u64)a - b - FQ_CC; FQ_CC = (u32)(s >> 32) & 1; return (u32)s;
+  u64 s = (u64)a - b - FQ_CIN(CK_SUBC_CC, (u64)a - b); FQ_CC = (u32)(s >> 32) & 1; return (u32)s;
 #else
   u32 r; asm volatile("subc.cc.u32 %0, %1, %2;" : "=r"(r) : "r"(a), "r"(b)); return r;
 #endif
 }
-FQ_FN u32 subc(u32 a, u32 b) {
+FQ_FN u32 subc(u32 a, u32 b FQ_SITE) {
 #ifdef FQ_HOSTSIM
-  return a - b - FQ_CC;
+  return a - b - FQ_CIN(CK_SUBC, (u64)a - b);
 #else
   u32 r; asm volatile("subc.u32 %0, %1, %2;" : "=r"(r) : "r"(a), "r"(b)); return r;
 #endif
@@ -96,33 +119,33 @@ FQ_FN void mul_wide(u32& lo, u32& hi, u32 a, u32 b) {
 #endif
 }
 // c + lo(a*b), carry out
-FQ_FN u32 mad_lo_cc(u32 a, u32 b, u32 c) {
+FQ_FN u32 mad_lo_cc(u32 a, u32 b, u32 c FQ_SITE) {
 #ifdef FQ_HOSTSIM
-  u64 s = (u64)(u32)((u64)a * b) + c; FQ_CC = (u32)(s >> 32); return (u32)s;
+  u64 s = (u64)(u32)((u64)a * b) + c; FQ_START(CK_MAD_LO_CC, s); FQ_CC = (u32)(s >> 32); return (u32)s;
 #else
   u32 r; asm volatile("mad.lo.cc.u32 %0, %1, %2, %3;" : "=r"(r) : "r"(a), "r"(b), "r"(c)); return r;
 #endif
 }
 // c + lo(a*b) + carry in, carry out
-FQ_FN u32 madc_lo_cc(u32 a, u32 b, u32 c) {
+FQ_FN u32 madc_lo_cc(u32 a, u32 b, u32 c FQ_SITE) {
 #ifdef FQ_HOSTSIM
-  u64 s = (u64)(u32)((u64)a * b) + c + FQ_CC; FQ_CC = (u32)(s >> 32); return (u32)s;
+  u64 t = (u64)(u32)((u64)a * b) + c, s = t + FQ_CIN(CK_MADC_LO_CC, t); FQ_CC = (u32)(s >> 32); return (u32)s;
 #else
   u32 r; asm volatile("madc.lo.cc.u32 %0, %1, %2, %3;" : "=r"(r) : "r"(a), "r"(b), "r"(c)); return r;
 #endif
 }
 // c + hi(a*b) + carry in, carry out
-FQ_FN u32 madc_hi_cc(u32 a, u32 b, u32 c) {
+FQ_FN u32 madc_hi_cc(u32 a, u32 b, u32 c FQ_SITE) {
 #ifdef FQ_HOSTSIM
-  u64 s = (u64)(u32)(((u64)a * b) >> 32) + c + FQ_CC; FQ_CC = (u32)(s >> 32); return (u32)s;
+  u64 t = (u64)(u32)(((u64)a * b) >> 32) + c, s = t + FQ_CIN(CK_MADC_HI_CC, t); FQ_CC = (u32)(s >> 32); return (u32)s;
 #else
   u32 r; asm volatile("madc.hi.cc.u32 %0, %1, %2, %3;" : "=r"(r) : "r"(a), "r"(b), "r"(c)); return r;
 #endif
 }
 // c + hi(a*b) + carry in (chain end)
-FQ_FN u32 madc_hi(u32 a, u32 b, u32 c) {
+FQ_FN u32 madc_hi(u32 a, u32 b, u32 c FQ_SITE) {
 #ifdef FQ_HOSTSIM
-  return (u32)(((u64)a * b) >> 32) + c + FQ_CC;
+  u64 t = (u64)(u32)(((u64)a * b) >> 32) + c; return (u32)(t + FQ_CIN(CK_MADC_HI, t));
 #else
   u32 r; asm volatile("madc.hi.u32 %0, %1, %2, %3;" : "=r"(r) : "r"(a), "r"(b), "r"(c)); return r;
 #endif

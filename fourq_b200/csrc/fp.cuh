@@ -148,12 +148,6 @@ FQ_FN fpw facc_merge(const facc& A) {
   r.w[4] = addc_cc(A.e4, A.o4); r.w[5] = addc(A.o5, 0);
   return r;
 }
-FQ_FN fpw fpw_add(const fpw& a, const fpw& b) {
-  fpw r;
-  r.w[0] = add_cc(a.w[0], b.w[0]); r.w[1] = addc_cc(a.w[1], b.w[1]); r.w[2] = addc_cc(a.w[2], b.w[2]);
-  r.w[3] = addc_cc(a.w[3], b.w[3]); r.w[4] = addc_cc(a.w[4], b.w[4]); r.w[5] = addc(a.w[5], b.w[5]);
-  return r;
-}
 // a - b, caller guarantees a >= b
 FQ_FN fpw fpw_sub(const fpw& a, const fpw& b) {
   fpw r;
