@@ -10,7 +10,7 @@ LIB_PATH = os.path.join(_HERE, "libfourq_b200.so")
 
 FQ_OK, FQ_ERR_NO_DEVICE, FQ_ERR_CUDA, FQ_ERR_ARG = 0, -1, -2, -3
 
-# op codes of fq_dev_run (include/fourq_b200.h)
+# op codes of fq_dev_run and fq_stream_run (include/fourq_b200.h)
 FPOP = {"mul": 0, "sqr": 1, "inv": 2, "add": 3, "sub": 4, "neg": 5, "invsqrt": 6}      # FQ_FP_* of the header
 DEVOP = {"fp_mul": 32, "fp_sqr": 33, "fp_inv": 34, "fp_add": 35, "fp_sub": 36, "fp_neg": 37, "fp_invsqrt": 38,
          "fp2_mul": 0, "fp2_sqr": 1, "fp2_inv": 2, "fp2_add": 3, "fp2_sub": 4, "fp2_neg": 5, "fp2_conj": 6, "fp2_invsqrt": 7, "fp2_select": 8, "fp_select": 9,
@@ -61,6 +61,7 @@ def bind(L):
         "fq_base_create": ([vp, i, vp, ctypes.POINTER(vp)], i), "fq_base_destroy": ([vp], i),
         "fq_dh_fixed": ([vp, vp, vp, vp, sz, i], i), "fq_mul_fixed": ([vp, vp, vp, sz, i], i),
         "fq_base_dev_run": ([vp, i, i, vp, vp, vp, sz, i, ctypes.POINTER(ctypes.c_float)], i),
+        "fq_stream_run": ([i, vp, vp, vp, vp, vp, sz, vp], i), "fq_base_stream_run": ([vp, i, vp, vp, vp, sz, vp], i),
         "fq_host_alloc": ([ctypes.POINTER(vp), sz], i), "fq_host_free": ([vp], i),
         "fq_host_alloc_sliced": ([ctypes.POINTER(vp), sz, sz, i], i), "fq_device_numa_node": ([i], i),
         "fq_dev_alloc": ([i, ctypes.POINTER(vp), sz], i), "fq_dev_free": ([i, vp], i),
@@ -81,7 +82,8 @@ EXPORTS = ["fq_version", "fq_device_count", "fq_last_error", "fq_set_device_base
            "fq_dh", "fq_dh_affine", "fq_dh_base", "fq_mul_base", "fq_dh_endo", "fq_dh_endo_affine", "fq_dh_endo_base",
            "fq_mul_endo_base", "fq_dh_base_comb", "fq_mul_base_comb", "fq_base_create", "fq_base_destroy", "fq_dh_fixed", "fq_mul_fixed",
            "fq_base_dev_run", "fq_x25519", "fq_host_alloc", "fq_host_free", "fq_host_alloc_sliced", "fq_device_numa_node",
-           "fq_dev_alloc", "fq_dev_free", "fq_dev_upload", "fq_dev_download", "fq_dev_run", "fq_dev_run3", "fq_dev_last_phase_ms", "fq_dev_flush_l2", "fq_imad_peak"]
+           "fq_dev_alloc", "fq_dev_free", "fq_dev_upload", "fq_dev_download", "fq_dev_run", "fq_dev_run3", "fq_dev_last_phase_ms", "fq_dev_flush_l2", "fq_imad_peak",
+           "fq_stream_run", "fq_base_stream_run"]
 
 
 def check(rc):

@@ -35,6 +35,7 @@
 #include <utility>
 #ifdef FQ_MOCK_CUDA
 #include "mock_cuda_runtime.h"
+#include "mock_cuda_stream.h"
 #else
 #include <cuda_runtime.h>
 #endif
@@ -53,6 +54,8 @@ extern cudaError_t fqk_comb_build(const void* xy, void** tabs_out, cudaStream_t 
 struct fq_base {
   uint8_t xy[64];
   mutable void* tabs[16] = {};        // one entry per device (kMaxDev)
+  // per device: the tables exist and stream calls may read tabs[dev] without DevCtx::mu (set once, after the build)
+  mutable std::atomic<bool> stream_ready[16] = {};
 };
 
 namespace {
@@ -331,6 +334,10 @@ struct DevCtx {
   std::mutex smu; std::condition_variable scv; std::deque<Chunk> chunks;
   CopyHelper copy_in, copy_out;   // staging copies of the feeder / of the drainer
   std::atomic<double> rate[3];    // rows per ms this GPU sustained in its last big calls, per class of operation (rate_class); 0 = unknown
+  // stream entry points: the scratch pool (created under mu) and whether ctx_init and the pool are done.  Once stream_ready is
+  // set, stream calls read comb, sms and pool without mu, so they never wait behind a host call's slice job.
+  cudaMemPool_t pool = nullptr;
+  std::atomic<bool> stream_ready{false};
   DevCtx() { for (auto& x : rate) x.store(0.0); }
 };
 DevCtx* g_ctx = nullptr;          // kMaxDev contexts, allocated once and never destroyed (their threads are detached)
@@ -781,6 +788,138 @@ int dev_run(const fq_base* base, int op, int dev, const void* a, const void* b, 
   return FQ_OK;
 }
 
+// ---------------------------------------------------------------- stream entry points (fq_stream_run, fq_base_stream_run)
+// One operation enqueued on the caller's stream over device buffers of one GPU: validate, make the GPU ready once, then
+// scratch from the GPU's pool, the kernels, a wipe of the scratch and its release, all on that stream.  No lock, no
+// synchronisation and no cudaMalloc after the first call on a GPU, so the sequence can be captured into a CUDA graph.
+
+// alignment of operand rows of `wb` bytes, as their kernels access them: 32- and 64-byte rows with 256-bit accesses (kio.cuh),
+// 16-byte GF(p) rows with 128-bit ones (k_fp_op, k_select), status, condition and on-curve bytes one byte at a time
+size_t row_align(int wb) { return wb >= 32 ? 32 : (size_t)wb; }
+
+// [p, p + bytes) is device memory at both ends (as classify() looks at both ends) and of one GPU: *dev = that GPU
+bool device_range(const void* p, size_t bytes, int* dev) {
+  int d[2];
+  const void* ends[2] = {p, (const char*)p + bytes - 1};
+  for (int i = 0; i < 2; i++) {
+    cudaPointerAttributes at;
+    if (cudaPointerGetAttributes(&at, ends[i]) != cudaSuccess) { cudaGetLastError(); return false; }
+    if (at.type != cudaMemoryTypeDevice) return false;
+    d[i] = at.device;
+  }
+  *dev = d[0];
+  return d[0] == d[1];
+}
+bool overlaps(const void* p, size_t pb, const void* q, size_t qb) { return (uintptr_t)p < (uintptr_t)q + qb && (uintptr_t)q < (uintptr_t)p + pb; }
+
+// The first stream call on a GPU initialises its context and scratch pool, the first with a registered base there builds the
+// base's tables (ctx_init and base_tables return with the tables on the GPU).  That work synchronises the library's own
+// stream and allocates, which a capturing stream forbids: it is refused there.  Later calls only read the two flags.
+int stream_prepare(DevCtx& c, const fq_base* base, cudaStream_t s) {
+  const bool ctx_done = c.stream_ready.load(std::memory_order_acquire);
+  if (ctx_done && (!base || base->stream_ready[c.dev].load(std::memory_order_acquire))) return FQ_OK;
+  cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+  CU(cudaStreamIsCapturing(s, &cap));
+  if (cap != cudaStreamCaptureStatusNone)
+    return fail(FQ_ERR_ARG, "the first stream call on device %d%s initialises the GPU and cannot be captured: make one call on that GPU outside capture first",
+                c.dev, ctx_done ? " with this base" : "");
+  std::lock_guard<std::mutex> l(c.mu);
+  int rc = ctx_init(c);
+  if (rc != FQ_OK) return rc;
+  if (!c.pool) {
+    cudaMemPoolProps props;
+    memset(&props, 0, sizeof(props));
+    props.allocType = cudaMemAllocationTypePinned;
+    props.location.type = cudaMemLocationTypeDevice;
+    props.location.id = c.dev;
+    cudaMemPool_t pool = nullptr;
+    CU(cudaMemPoolCreate(&pool, &props));
+    uint64_t keep = UINT64_MAX;                                    // keep released blocks mapped between calls (fq_trim returns them)
+    cudaError_t e = cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &keep);
+    if (e != cudaSuccess) { cudaMemPoolDestroy(pool); return fail(FQ_ERR_CUDA, "setting the release threshold of the scratch pool failed: %s", cudaGetErrorString(e)); }
+    c.pool = pool;
+  }
+  c.stream_ready.store(true, std::memory_order_release);
+  if (base) {
+    if ((rc = base_tables(c, *base)) != FQ_OK) return rc;
+    base->stream_ready[c.dev].store(true, std::memory_order_release);
+  }
+  return FQ_OK;
+}
+
+// on the current device `dev`, after validation
+int stream_enqueue(const OpDesc& d, const fq_base* base, int dev, const void* a, const void* b, const void* cbuf, void* out, void* status, size_t n, cudaStream_t s) {
+  DevCtx& c = ctx_of(dev);
+  int rc = stream_prepare(c, base, s);
+  if (rc != FQ_OK) return rc;
+  // Scratch from the pool, ordered on the caller's stream: concurrent streams never share it, and a capturing stream records
+  // allocation nodes.  It holds tables of secret multiples and pool memory can go back to any allocation of the process
+  // (fq_trim), so it is always zeroed before it is released.
+  const size_t sb = scratch_bytes(d.scratch, n);
+  void* scratch = nullptr;
+  if (sb) CU(cudaMallocFromPoolAsync(&scratch, sb, c.pool, s));
+  const cudaError_t e = launch(c, d.op, base ? base->tabs[dev] : nullptr, a, b, cbuf, out, status, n, s, scratch);
+  if (sb) {
+    const cudaError_t ez = cudaMemsetAsync(scratch, 0, sb, s), ef = cudaFreeAsync(scratch, s);
+    if (e == cudaSuccess) { CU(ez); CU(ef); }
+  }
+  if (e != cudaSuccess) return fail(FQ_ERR_CUDA, "launch of operation %d on device %d failed: %s", d.op, dev, cudaGetErrorString(e));
+  return FQ_OK;
+}
+
+int stream_run(const fq_base* base, int op, const void* a, const void* b, const void* cbuf, void* out, void* status, size_t n, void* stream) {
+#ifdef FQ_MOCK_CUDA
+  if (!cudaMallocFromPoolAsync) return fail(FQ_ERR_CUDA, "this mock build has no stream runtime (tests/hostsim/mock_cuda_stream.cpp)");
+#endif
+  const OpDesc d = describe(op);
+  if (d.op < 0) return fail(FQ_ERR_ARG, "unknown operation %d", op);
+  if (n == 0) return FQ_OK;
+  static const char* const names[kOperands] = {"a", "b", "c", "out", "status"};
+  const void* ptrs[kOperands] = {a, b, cbuf, out, status};
+  for (int w = 0; w < kOperands; w++) if (operand_bytes(d, w) && !ptrs[w]) return fail(FQ_ERR_ARG, "null operand %s", names[w]);
+  const int count = device_count();
+  if (count < 0) return count;
+  int dev = -1;
+  for (int w = 0; w < kOperands; w++) {
+    const int wb = operand_bytes(d, w);
+    if (!wb) continue;
+    int dw = -1;
+    if (!device_range(ptrs[w], n * wb, &dw)) return fail(FQ_ERR_ARG, "operand %s (%zu rows of %d bytes) is not device memory of one GPU", names[w], n, wb);
+    if (dev >= 0 && dw != dev) return fail(FQ_ERR_ARG, "operand %s is on device %d, operand a on device %d: a stream call runs on one GPU", names[w], dw, dev);
+    dev = dw;
+    if ((uintptr_t)ptrs[w] % row_align(wb)) return fail(FQ_ERR_ARG, "operand %s is not %zu-byte aligned (rows of %d bytes)", names[w], row_align(wb), wb);
+  }
+  if (dev < 0 || dev >= count) return fail(FQ_ERR_ARG, "device %d out of range (%d device(s))", dev, count);
+  // An output may be exactly an input of its own row width (every kernel reads a row before it writes that row, and the DH
+  // ops read k and the point in k_dh_prep before k_dh_finish writes); the batched inversions park prefix products in out.
+  const bool parks_in_out = op == FQ_DEVOP_FP2_INV || op == FQ_DEVOP_F25519_BASE + FQ_FP_INV;
+  for (int o = 3; o < kOperands; o++) {
+    const int ob = operand_bytes(d, o);
+    for (int w = 0; ob && w < kOperands; w++) {
+      const int wb = operand_bytes(d, w);
+      if (w == o || !wb || !overlaps(ptrs[o], n * ob, ptrs[w], n * wb)) continue;
+      if (w < 3 && ptrs[o] == ptrs[w] && ob == wb && !parks_in_out) continue;
+      return fail(FQ_ERR_ARG, "operand %s overlaps operand %s%s", names[o], names[w], parks_in_out && ptrs[o] == ptrs[w] ? " (inv: out must not alias a, the prefix products are parked in out)" : "");
+    }
+  }
+  // The legacy default stream (NULL) is the one of the device made current below.  CUDA refuses cudaStreamGetDevice on a
+  // capturing stream, and the refusal invalidates the capture: a captured call relies on the check of the calls outside capture.
+  cudaStream_t s = (cudaStream_t)stream;
+  if (s) {
+    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+    CU(cudaStreamIsCapturing(s, &cap));
+    int sd = dev;
+    if (cap == cudaStreamCaptureStatusNone) CU(cudaStreamGetDevice(s, &sd));
+    if (sd != dev) return fail(FQ_ERR_ARG, "the stream belongs to device %d, the buffers to device %d", sd, dev);
+  }
+  int prev = 0;
+  CU(cudaGetDevice(&prev));
+  CU(cudaSetDevice(dev));
+  const int rc = stream_enqueue(d, base, dev, a, b, cbuf, out, status, n, s);
+  cudaSetDevice(prev);
+  return rc;
+}
+
 }  // namespace
 
 extern "C" {
@@ -809,6 +948,7 @@ int fq_trim(void) {
     CU(cudaDeviceSynchronize());
     for (int si = 0; si < kSlots; si++) { int rc = slot_wipe_free(c.slot[si]); if (rc != FQ_OK) return rc; }
     if (c.flush) { CU(cudaFree(c.flush)); c.flush = nullptr; }
+    if (c.pool) CU(cudaMemPoolTrimTo(c.pool, 0));        // stream-call scratch: every block was zeroed before it was freed
   }
   return FQ_OK;
 }
@@ -904,6 +1044,15 @@ int fq_mul_fixed(const fq_base* base, const uint8_t* k, uint8_t* enc_out, size_t
 int fq_base_dev_run(const fq_base* base, int dh, int dev, const void* k, void* out, void* status, size_t n, int iters, float* ms) {
   if (!base) return fail(FQ_ERR_ARG, "null base");
   return dev_run(base, dh ? kOpDhFixed : kOpMulFixed, dev, k, nullptr, nullptr, out, dh ? status : nullptr, n, iters, ms);
+}
+
+int fq_stream_run(int op, const void* a, const void* b, const void* c, void* out, void* status, size_t n, void* stream) {
+  if (op == kOpDhFixed || op == kOpMulFixed) return fail(FQ_ERR_ARG, "unknown operation %d", op);      // need a base: fq_base_stream_run
+  return stream_run(nullptr, op, a, b, c, out, status, n, stream);
+}
+int fq_base_stream_run(const fq_base* base, int dh, const void* k, void* out, void* status, size_t n, void* stream) {
+  if (!base) return fail(FQ_ERR_ARG, "null base");
+  return stream_run(base, dh ? kOpDhFixed : kOpMulFixed, k, nullptr, nullptr, out, dh ? status : nullptr, n, stream);
 }
 
 int fq_host_alloc(void** p, size_t bytes) {

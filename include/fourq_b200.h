@@ -181,7 +181,8 @@ FQ_API int fq_mul_fixed(const fq_base* base, const uint8_t* k, uint8_t* enc_out,
 FQ_API int fq_x25519(const uint8_t* k, const uint8_t* u, uint8_t* out, size_t n, int ndev);
 
 /* Frees the staging and scratch buffers the engine keeps per GPU between calls (up to ~0.5 GB per stream slot for the DH
- * ops); contexts, streams and the fixed-base tables stay.  The next call allocates what it needs again. */
+ * ops) and trims the scratch pool of the stream entry points (up to ~4.9 GB per GPU, fq_stream_run) to zero; contexts,
+ * streams and the fixed-base tables stay.  The next call allocates what it needs again. */
 FQ_API int fq_trim(void);
 
 /* ---- pinned host memory for zero-staging transfers (optional; any host pointer is accepted above) */
@@ -237,6 +238,38 @@ FQ_API int fq_dev_last_phase_ms(float* ms3);
 /* fq_dh_fixed (dh = 1) or fq_mul_fixed (dh = 0) on device buffers of GPU `dev`, `iters` launches as fq_dev_run (the first
  * call on a GPU builds the base's tables there before timing); status may be NULL for dh = 0 */
 FQ_API int fq_base_dev_run(const fq_base* base, int dh, int dev, const void* k, void* out, void* status, size_t n, int iters, float* ms);
+/* ---- stream-ordered entry points, for batches that already sit in GPU memory (a PyTorch job, inputs built by the caller's
+ * own kernels).  The operation is enqueued on `stream` (a cudaStream_t; NULL = the legacy default stream) and the call
+ * returns without waiting: the results are there once the stream reaches that point.
+ *   - op is an FQ_DEVOP_* code with the operands of fq_dev_run3 above.  Outputs, statuses and the zero fill of failed rows
+ *     are byte for byte those of the host entry point; rows past n are not written.  Table selection follows
+ *     fq_set_select_mode.
+ *   - Every operand must be device memory of one GPU (both ends of each range are checked), and a non-NULL stream must
+ *     belong to that GPU (checked on calls outside capture: CUDA does not name the device of a capturing stream).  The call makes that GPU current and restores the calling thread's device before it returns;
+ *     fq_set_device_base and ndev play no part.
+ *   - Refused with FQ_ERR_ARG before anything is enqueued, outputs untouched: an unknown op; a NULL operand the op needs;
+ *     an operand that is not device memory of that GPU; a stream of another GPU; a row operand that is not aligned as
+ *     its kernel accesses it (32 bytes for rows of 32 and 64 bytes, 16 for GF(p) rows: an offset view of a tensor is the
+ *     usual way to get this wrong); an output that overlaps an input other than as an exact alias of the same row width,
+ *     or overlaps the other output (FQ_DEVOP_FP2_INV and the GF(2^255-19) inversion refuse even the exact alias: they park
+ *     prefix products in out); for fq_base_stream_run a NULL base.  n == 0 returns FQ_OK and enqueues nothing.
+ *   - Scratch (the DH ops, the fixed-base ops, X25519) comes from a memory pool the library keeps per GPU, allocated,
+ *     zeroed and released on the caller's stream around the kernels: no workspace argument, and concurrent streams never
+ *     share scratch.  The pool keeps up to ~4.9 GB per GPU mapped between calls (the scratch of one 2^22-row DH launch
+ *     group) until fq_trim.
+ *   - The first stream call on a GPU initialises the GPU (constant and comb tables, the pool), and the first with a base
+ *     builds that base's tables there; both wait for the library's own stream once.  A first call on a stream that is
+ *     being captured is therefore refused with FQ_ERR_ARG: make one call on that GPU outside capture first.  After that a
+ *     call makes no synchronising call, no cudaMalloc / cudaFree and no event record, and takes no lock a host call
+ *     holds, so it does not wait behind host calls on the same GPU and can be captured into a CUDA graph (the scratch
+ *     becomes graph allocation nodes).
+ *   - Statuses stay on the device: checking them on the host is the caller's synchronisation.
+ *   - fq_base_destroy must not run while stream work that uses the base is pending, and a graph that captured such a call
+ *     must not be replayed after the base is destroyed. */
+FQ_API int fq_stream_run(int op, const void* a, const void* b, const void* c, void* out, void* status, size_t n, void* stream);
+/* fq_dh_fixed (dh = 1) / fq_mul_fixed (dh = 0, status unused) of a registered base, the same way */
+FQ_API int fq_base_stream_run(const fq_base* base, int dh, const void* k, void* out, void* status, size_t n, void* stream);
+
 /* writes `bytes` of zeros over a scratch buffer larger than L2 (used between timed iterations) */
 FQ_API int fq_dev_flush_l2(int dev);
 
